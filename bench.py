@@ -2,13 +2,17 @@
 """bench.py -- P(k) pipeline throughput (deposit + r2c FFT + shell binning) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one complete P(k) of one synthetic particle set: deposit (sort + tiled deposit;
 twice when interlaced), r2c FFT(s), fused binning, result on the host.  Prints ONE JSON line.
+--dump-outputs DIR writes the result of the last timed step as DIR/<name>.npy (float64; complex
+arrays as <name>_real and <name>_imag).  The inputs are generated from fixed seeds, so two builds
+run with the same arguments can be compared output for output.
 
 Workloads (BASELINE.json configs):
   c3  1024^3 Zel'dovich particles, TSC + interlacing + window compensation, 1024^3 mesh  -- the
-      configuration the metric is quoted on; default when the device has the memory for it
+      configuration the metric is quoted on; the default
   c2  512^3 Zel'dovich particles, CIC, 512^3 mesh
   c1  128^3 uniform particles, CIC, 128^3 mesh (the reference's CPU-runnable case)
 Inputs are far larger than L2 (126 MB), so no explicit L2 flush is needed between steps.
@@ -24,6 +28,7 @@ import signal
 import statistics
 import subprocess
 import sys
+import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -52,6 +57,7 @@ WORKLOADS["c4s"] = dict(WORKLOADS["c4"], n=512, mesh=512, halos=125000,
 WORKLOADS["c2u"] = dict(WORKLOADS["c2"], kind="uniform", name="c2u: 512^3 uniform-random particles (incoherent order), CIC, 512^3 mesh")
 METRIC = "P(k) pipeline Mparticles/s (deposit+FFT+binning)"
 UNIT = "Mparticles/s"
+HBM_PEAK_GBS = 6535.4       # denominator of the roofline fractions: HBM copy bandwidth measured on a B200 (BASELINE.md)
 
 
 def make_particles(wl: dict, dev, x_planes=None, rank: int = 0, world: int = 1):
@@ -89,6 +95,20 @@ def golden_check(wl_key: str, res: dict, rtol: float = 1e-4):
            "max_rel_k": float(relk.max()), "rtol": rtol, "bins": int(ok.sum())}
     out["ok"] = bool(modes_equal and out["max_rel_P"] <= rtol and out["max_rel_k"] <= 1e-12)
     return out
+
+
+def dump_outputs(res: dict, out_dir: str) -> None:
+    """Writes every numeric array of a step's result (k, power, modes, edges, Nsum; the slab path adds total_mass) as
+    <out_dir>/<name>.npy in float64, complex arrays as <name>_real and <name>_imag.  A few kB per workload: the result
+    has one entry per k shell."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, value in res.items():
+        a = np.asarray(value)
+        if a.dtype.kind not in "biufc":
+            continue
+        parts = {name + "_real": a.real, name + "_imag": a.imag} if a.dtype.kind == "c" else {name: a}
+        for part, arr in parts.items():
+            np.save(os.path.join(out_dir, part + ".npy"), arr.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------
@@ -227,7 +247,8 @@ class ClockSampler:
          "clocks_event_reasons.sw_power_cap")
 
     def __init__(self, gpu_index: int):
-        self.idx, self.proc, self.path = gpu_index, None, f"/tmp/apk_clocks_{os.getpid()}.csv"
+        self.idx, self.proc = gpu_index, None
+        self.path = os.path.join(tempfile.gettempdir(), f"apk_clocks_{os.getpid()}.csv")
 
     def start(self):
         try:
@@ -506,13 +527,8 @@ def run_ours(args, wl_key: str) -> None:
         return
 
     # ---------------- roofline of the dominant hand-written kernel ---------------------------
-    peaks = {}
-    try:
-        peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
-    except Exception:
-        pass
-    peak = float(peaks.get("hbm_gbs", 6650.0))
-    peak_src = "measured (MEASURED_PEAKS.json hbm_gbs)" if "hbm_gbs" in peaks else "fallback 6650 GB/s (B200_PROFILING.md)"
+    peak = HBM_PEAK_GBS
+    peak_src = "measured HBM copy bandwidth of a B200 (BASELINE.md)"
     traffic = {}
     try:                                            # DRAM bytes per launch from the committed ncu --set full capture
         traffic = json.load(open(os.path.join(ROOT, "profiles", "ncu_traffic.json"))).get(wl_key, {})
@@ -623,6 +639,8 @@ def run_ours(args, wl_key: str) -> None:
     if routing_stress is not None:
         out["routing_stress"] = routing_stress
     print(json.dumps(out), flush=True)
+    if args.dump_outputs:
+        dump_outputs(res, args.dump_outputs)
     if world > 1:
         dist.destroy_process_group()
     bad = [c for c in (check, e2e_check) if c is not None and not c["ok"]]
@@ -632,18 +650,12 @@ def run_ours(args, wl_key: str) -> None:
 
 
 def pick_workload(args) -> str:
+    """The workload follows from the arguments alone (not from the device's free memory), so the same arguments always
+    run, and --dump-outputs writes, the same computation."""
     if args.workload:
         return args.workload
     if args.impl == "reference":
         return os.environ.get("APK_BENCH_WORKLOAD", "c3")
-    try:
-        import torch
-        if torch.cuda.is_available():
-            free, total = torch.cuda.mem_get_info(int(os.environ.get("LOCAL_RANK", "0")))
-            world = int(os.environ.get("WORLD_SIZE", "1"))
-            return "c3" if free > 60e9 / world + 20e9 else "c2"
-    except Exception:
-        pass
     return "c3"
 
 
@@ -660,7 +672,13 @@ def main():
                     help="diagnostic (N = 1): reorder the particle set on the device before the run -- 'cell' = sorted by mesh "
                          "cell (z fastest), 'random' = shuffled; the golden check still applies (P(k) does not depend on order)")
     ap.add_argument("--no-routing-stress", action="store_true", help="N > 1: skip the unsorted-input run after the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm times a sample of the workload, not a whole P(k)")
     # whole-run watchdog: a dead-lock (collectives, device-side barriers) must not hold the GPUs for long
     limit = int(os.environ.get("APK_BENCH_TIME_LIMIT_S", "1500"))
     if limit > 0 and hasattr(signal, "SIGALRM"):
@@ -678,4 +696,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the bench writes nothing into the tree it runs from (it may be read-only)
     main()

@@ -64,6 +64,27 @@ def test_missing_library_is_an_error(monkeypatch, tmp_path):
         _lib.load()
 
 
+def test_bench_dump_outputs_writes_every_result_array(tmp_path):
+    import bench
+    res = {"k": np.array([0.1, np.nan]), "power": np.array([2.0 + 1.0j, 3.0 + 0.0j]), "modes": np.array([6, 0]),
+           "edges": np.array([0.0, 0.2, 0.4]), "Nsum": np.array([1, 6, 0, 2], dtype=np.int64)}
+    bench.dump_outputs(res, str(tmp_path / "out"))
+    got = {p.stem: np.load(p) for p in (tmp_path / "out").iterdir()}
+    assert set(got) == {"k", "power_real", "power_imag", "modes", "edges", "Nsum"}
+    assert all(a.dtype == np.float64 for a in got.values())
+    np.testing.assert_array_equal(got["k"], res["k"])
+    np.testing.assert_array_equal(got["power_real"] + 1j * got["power_imag"], res["power"])
+    np.testing.assert_array_equal(got["Nsum"], res["Nsum"])
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_rejects_arguments_it_cannot_honour(argv):
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True)
+    assert out.returncode == 2 and "bench.py: error" in out.stderr
+
+
 def test_recorded_bench_lines_carry_the_contract_keys():
     """The JSON lines bench.py printed on the GPU box at the end of the round (committed under profiles/) have every key the
     measurement contract names -- a guard against a bench change that drops one (the bench itself needs a GPU)."""
