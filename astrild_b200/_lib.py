@@ -60,6 +60,13 @@ SIGNATURES = {
     "apk_kmu_create": [ct.POINTER(_vp), _vp, _i, _i, _i] + [_vp] * 5 + [_i, _i, _vp, _i, _vp] + [_vp] * 6 + [_i, _i],
     "apk_kmu_destroy": [_vp],
     "apk_kmu_bin": [_vp] * 11,
+    "apk_bispec_create": [ct.POINTER(_vp), _vp, _d, _d, _d, _i, _i, _i],
+    "apk_bispec_destroy": [_vp],
+    "apk_bispec_triples": [_vp, _vp, _i, ct.POINTER(_i)],
+    "apk_bispec_scratch_bytes": [_vp, ct.POINTER(_sz)],
+    "apk_bispec_count": [_vp, _vp, _sz, _vp, ct.POINTER(_d), _vp],
+    "apk_bispec_measure": [_vp, _vp, _vp, _vp, _sz, _vp, _vp],
+    "apk_bispec_last_ms": [_vp, ct.POINTER(ct.c_float)],
     "apk_assign_grid": [_vp, _vp, _vp, _vp, _i, _vp, _i, _i64, _vp, _vp, _vp, _vp],
     "apk_gather_records": [_vp, _vp, _i64, _vp, _i, _vp],
     "apk_tables_k_axis": [_i, _d, _i, _vp],

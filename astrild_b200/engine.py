@@ -59,6 +59,19 @@ class Binning:
 
 
 @dataclass
+class BispecBinning:
+    handle: ct.c_void_p
+    edges: np.ndarray
+    triples: np.ndarray          # (ntriples, 3) int32: the kept (i, j, l), i <= j <= l
+    scratch_bytes: int
+    key: tuple
+    dk: float
+    kmax: float
+    ntri: np.ndarray | None = None
+    residual: float | None = None
+
+
+@dataclass
 class KmuBinning:
     handle: ct.c_void_p
     edges: np.ndarray
@@ -92,7 +105,10 @@ class PkEngine:
     def close(self) -> None:
         if self._plan:
             for b in self._binnings.values():
-                (self.lib.apk_kmu_destroy if isinstance(b, KmuBinning) else self.lib.apk_binning_destroy)(b.handle)
+                if isinstance(b, BispecBinning):
+                    self.lib.apk_bispec_destroy(b.handle)
+                else:
+                    (self.lib.apk_kmu_destroy if isinstance(b, KmuBinning) else self.lib.apk_binning_destroy)(b.handle)
             self._binnings.clear()
             self.lib.apk_plan_destroy(self._plan)
             self._plan = ct.c_void_p()
@@ -518,3 +534,78 @@ class PkEngine:
 
     def bin_power(self, binning: Binning, c1, c1s=None, c2=None, c2s=None, scale: float = 1.0) -> dict:
         return self.finish(self.bin_power_raw(binning, c1, c1s, c2, c2s), binning, scale)
+
+    # ------------------------------------------------------------------ bispectrum (FFT estimator)
+    def bispec_binning(self, kmin: float = 0.0, dk: float | None = None, kmax: float | None = None,
+                       compensation: tuple | None = None, interlaced: bool = False, k_dtype=np.float64) -> "BispecBinning":
+        """Shells and kept triples of a bispectrum (apk_bispec_create): dk defaults to 2 pi / L, kmax to (2/3) pi N / L.
+        Cached like the other binnings; it owns the triangle counts once ``bispec_counts`` has computed them."""
+        if self.n0 != self.N:
+            raise AstrildPkError("the bispectrum runs on single-GPU engines only (no slab path)")
+        dk = 2 * np.pi / self.L if dk is None else float(dk)
+        kmax = 2.0 / 3.0 * np.pi * self.N / self.L if kmax is None else float(kmax)
+        key = ("bispec", float(kmin), dk, kmax, compensation, bool(interlaced), np.dtype(k_dtype).str)
+        got = self._binnings.get(key)
+        if got is not None:
+            return got
+        rs = 0 if compensation is None else _lib.RESAMPLERS[str(compensation[0]).lower()]
+        handle = ct.c_void_p()
+        _lib.call("apk_bispec_create", ct.byref(handle), self._plan, float(kmin), dk, kmax,
+                  _lib.APK_F32 if np.dtype(k_dtype) == np.float32 else _lib.APK_F64, rs, int(bool(interlaced)))
+        try:
+            nt = ct.c_int()
+            _lib.call("apk_bispec_triples", handle, None, 0, ct.byref(nt))
+            ijl = np.zeros((max(nt.value, 1), 3), dtype=np.int32)
+            _lib.call("apk_bispec_triples", handle, ijl.ctypes.data_as(ct.c_void_p), nt.value, ct.byref(nt))
+            need = ct.c_size_t()
+            _lib.call("apk_bispec_scratch_bytes", handle, ct.byref(need))
+        except Exception:
+            self.lib.apk_bispec_destroy(handle)
+            raise
+        got = BispecBinning(handle, tables.k_edges(self.N, self.L, kmin, dk, kmax), ijl[:nt.value].copy(), need.value,
+                            key, dk, kmax)
+        self._binnings[key] = got
+        return got
+
+    def bispec_counts(self, bk: "BispecBinning", scratch: torch.Tensor) -> np.ndarray:
+        """N_tri per kept triple (int64, host), computed once per binning in float64 on the device."""
+        if bk.ntri is None:
+            out = torch.empty(max(len(bk.triples), 1), dtype=torch.int64, device=self.device)
+            res = ct.c_double()
+            _lib.call("apk_bispec_count", bk.handle, _ptr(scratch), scratch.numel(), _ptr(out), ct.byref(res), self.stream)
+            bk.ntri = out[:len(bk.triples)].cpu().numpy().copy()
+            bk.residual = res.value
+        return bk.ntri
+
+    def bispec_raw(self, bk: "BispecBinning", scratch: torch.Tensor, c1, c1s=None) -> torch.Tensor:
+        """T_F = sum_x F_i F_j F_l per kept triple, float64 on the device."""
+        out = torch.empty(max(len(bk.triples), 1), dtype=torch.float64, device=self.device)
+        _lib.call("apk_bispec_measure", bk.handle, _ptr(c1), _ptr(c1s), _ptr(scratch), scratch.numel(), _ptr(out),
+                  self.stream)
+        return out[:len(bk.triples)]
+
+    def last_bispec_ms(self, bk: "BispecBinning") -> dict:
+        ms = (ct.c_float * 4)()
+        _lib.call("apk_bispec_last_ms", bk.handle, ms)
+        return {"fill": ms[0], "c2r": ms[1], "reduce": ms[2], "fold": ms[3]}
+
+    def bispectrum(self, bk: "BispecBinning", tsum, power: dict, field_scale: float, shot: float) -> dict:
+        """Raw sums (device or host) + the 1-D ``bin_power`` result of the same edges -> host arrays, triples with no
+        triangle dropped.  B = (L^6 s^3 / N^9) T_F / (N^3 N_tri); Bshot = shot (P1 + P2 + P3) - 2 shot^2 / mean (passed
+        in as ``shot`` = (S, mean) or NaN / 0)."""
+        t = tsum.cpu().numpy() if isinstance(tsum, torch.Tensor) else np.asarray(tsum, dtype=np.float64)
+        ntri = bk.ntri
+        keep = ntri > 0
+        ijl = bk.triples[keep]
+        N, L = float(self.N), self.L
+        B = (L ** 6 * field_scale ** 3 / N ** 9) * t[keep] / (N ** 3 * ntri[keep].astype(np.float64))
+        k, P = power["k"], power["power"].real
+        P1, P2, P3 = P[ijl[:, 0]], P[ijl[:, 1]], P[ijl[:, 2]]
+        if isinstance(shot, tuple):
+            S, mean = shot
+            Bshot = (S * (P1 + P2 + P3) - 2.0 * S * S) / mean
+        else:
+            Bshot = np.full(len(ijl), float(shot))
+        return {"k1": k[ijl[:, 0]], "k2": k[ijl[:, 1]], "k3": k[ijl[:, 2]], "bins": ijl.astype(np.int64), "B": B,
+                "triangles": ntri[keep].copy(), "P1": P1, "P2": P2, "P3": P3, "Bshot": Bshot}
+

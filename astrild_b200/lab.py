@@ -306,3 +306,73 @@ class FFTPower:
 
     def run(self):
         return self.power, self.poles
+
+
+def _free_device_bytes(device) -> int:
+    """Bytes a new allocation can get on ``device``: free device memory plus what torch's allocator holds unused."""
+    free, _total = torch.cuda.mem_get_info(device)
+    return int(free) + int(torch.cuda.memory_reserved(device) - torch.cuda.memory_allocated(device))
+
+
+class FFTBispectrum:
+    """Bispectrum B(k1, k2, k3) of one field: ``FFTBispectrum(first, kmin=0., dk=None, kmax=None)``.
+
+    ``first`` is a CatalogMesh or an ArrayMesh, as for FFTPower.  Shells are the 1-D bins of the same edges
+    (dk = 2 pi / L and kmax = (2/3) pi N / L by default: no triangle is aliased then; kmax may go up to the Nyquist
+    wavenumber, and the estimator then also counts triangles that close modulo the grid).  The FFT estimator runs on the
+    device: shell fields F_b = c2r of the field masked to shell b, B = V^2 <delta delta delta> =
+    (L^6 s^3 / N^9) sum_x F_i F_j F_l / (N^3 N_tri), with N_tri the exact number of ordered triangles (q1, q2, q3) of
+    the three shells, computed once in float64 and cached.
+
+    ``self.bispectrum`` is a BinnedStatistic over one ``triangle`` dimension (triples i <= j <= l with at least one
+    triangle) with variables ``k1 k2 k3`` (mean |k| of each shell), ``bins`` (i, j, l), ``B``, ``triangles`` (N_tri),
+    ``P1 P2 P3`` (the shells' P(k), shot noise not subtracted) and ``Bshot`` = S (P1 + P2 + P3) - 2 S^2 for the
+    Poisson shot noise S of the field's P(k) (divided by the mean density for an un-normalised field).  Bshot holds
+    for unit or scalar weights; it is 0 for an ArrayMesh and NaN for per-particle weights.  It is reported, never
+    subtracted.  Auto-bispectra of single-GPU meshes only; the scratch (the shell fields) must fit in free device
+    memory.
+    """
+
+    def __init__(self, first, kmin=0.0, dk=None, kmax=None, k_dtype=np.float64, second=None, third=None):
+        if (second is not None and second is not first) or (third is not None and third is not first):
+            raise AstrildPkError("FFTBispectrum computes auto-bispectra only: cross bispectra are not supported")
+        if getattr(first, "_fold", 0):
+            raise AstrildPkError("FFTBispectrum does not support folded boxes (fold > 0)")
+        eng = first._eng
+        if eng.n0 != eng.N:
+            raise AstrildPkError("FFTBispectrum runs on single-GPU meshes only (no slab path)")
+        N, L = eng.N, eng.L
+        (c1, c1s), s, comp = first._complex_fields()
+        bk = eng.bispec_binning(kmin, dk, kmax, comp, c1s is not None, k_dtype)
+        free = _free_device_bytes(eng.device)
+        if bk.scratch_bytes > free:
+            raise AstrildPkError(
+                f"FFTBispectrum needs {bk.scratch_bytes} bytes of device scratch for {len(bk.edges) - 1} shell fields, "
+                f"{free} are free: use a larger dk (fewer shells) or a smaller kmax")
+        scratch = torch.empty(bk.scratch_bytes, dtype=torch.uint8, device=eng.device)
+        eng.bispec_counts(bk, scratch)
+        tsum = eng.bispec_raw(bk, scratch, c1, c1s)
+        binning = eng.binning(kmin, bk.dk, bk.kmax, comp, c1s is not None, k_dtype)
+        power = eng.bin_power(binning, c1, c1s, None, None, L ** 3 * s * s / float(N) ** 6)
+        del scratch
+        if isinstance(first, CatalogMesh):
+            w = first._w
+            S = float(first.shotnoise)
+            if w is not None and not np.isscalar(w):
+                shot = float("nan")
+            else:
+                m = 1.0 if w is None else float(w)
+                mean = 1.0 if first._normalize else first._npart() * m / L ** 3
+                shot = (S, mean)
+        else:
+            S, shot = 0.0, 0.0
+        res = eng.bispectrum(bk, tsum, power, s, shot)
+        self.first = first
+        self.attrs = {"edges": bk.edges, "Nmesh": np.array([N] * 3), "BoxSize": np.array([L] * 3), "shotnoise": S,
+                      "kmin": kmin, "dk": bk.dk, "kmax": bk.kmax, "volume": L ** 3,
+                      "count_residual": bk.residual}
+        ntr = len(res["B"])
+        self.bispectrum = BinnedStatistic(["triangle"], [np.arange(ntr + 1)], res, dict(self.attrs))
+
+    def run(self):
+        return self.bispectrum

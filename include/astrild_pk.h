@@ -200,6 +200,32 @@ int apk_kmu_destroy(apk_kmu *kmu);
 int apk_kmu_bin(apk_kmu *kmu, const void *c1, const void *c1s, const void *c2, const void *c2s,
                 double *xsum, double *musum, double *ysum_re, double *ysum_im, int64_t *nsum, void *stream);
 
+/* ---- bispectrum B(k1, k2, k3) of one field (FFT estimator, exact triangle counts) ------------------------------ */
+/* Shells b = 0 .. Nb-1 are the bins of the 1-D binning of the same edges (apk_tables_k_edges(N, L, kmin, dk, kmax);
+ * dk <= 0: 2 pi / L; kmax <= 0: (2/3) pi N / L, which keeps every triangle free of aliasing; kmax above pi N / L is
+ * refused); the k = 0 mode is in no shell.  Nb is at most 128.  F_b(x) = un-normalised c2r of the k-grid masked to shell
+ * b; the triples are i <= j <= l minus those that provably hold no triangle (lo_l >= hi_i + hi_j and
+ * hi_i + hi_j + hi_l <= 2 k_Nyquist).  tsum = sum_x F_i F_j F_l, N_tri = (sum_x D_i D_j D_l) / N^3 with D_b the same for
+ * c == 1 (ordered (q1, q2, q3), q1 + q2 + q3 = 0 modulo the grid), and B = L^6 s^3 / N^9 * tsum / (N^3 N_tri) for a field
+ * scale s as in FFTPower.  resampler (APK_CIC / APK_TSC, 0 = no compensation) and interlaced select the window
+ * deconvolution and interlace-combine of apk_bin_power.  Single-GPU plans only.                                      */
+typedef struct apk_bispec apk_bispec;
+int apk_bispec_create(apk_bispec **bk, apk_plan *plan, double kmin, double dk, double kmax, int k_dtype,
+                      int resampler /* 0 = no compensation */, int interlaced);
+int apk_bispec_destroy(apk_bispec *bk);
+/* the kept triples (i, j, l) as ijl_host[3 t + 0..2]; ijl_host may be NULL to query the number                     */
+int apk_bispec_triples(const apk_bispec *bk, int *ijl_host, int capacity, int *ntriples); /* after the skip rule */
+int apk_bispec_scratch_bytes(const apk_bispec *bk, size_t *bytes);   /* max(f64 indicator fields, f32 fields) + cuFFT */
+/* N_tri per kept triple (DEVICE int64); computed once per object in float64 and cached.  Fails if a count is further
+ * than 0.1 from an integer (precision lost); residual_host (may be NULL) receives the largest |T_D / N^3 - N_tri|.
+ * Synchronises `stream`.                                                                                            */
+int apk_bispec_count(apk_bispec *bk, void *scratch, size_t bytes, int64_t *ntri_dev, double *residual_host, void *stream);
+/* tsum_dev (DEVICE float64 per kept triple) = sum_x F_i F_j F_l of the field c1 (complex64 k-grid after apk_fft_r2c) and
+ * its interlaced twin c1s (NULL unless created with interlaced != 0)                                                */
+int apk_bispec_measure(apk_bispec *bk, const void *c1, const void *c1s, void *scratch, size_t bytes,
+                       double *tsum_dev, void *stream);     /* c1 / c1s are read, never modified */
+int apk_bispec_last_ms(apk_bispec *bk, float ms[4]);       /* fill, c2r, reduction, fold (plan timing on) */
+
 /* ---- ingest (SURVEY.md section 8f, N1) ------------------------------------------------------------------- */
 /* PowerSpectrum3D._read_data's gridder (src/astrild/power_spectra/power_spectrum_3d.py:142-148):
  *   value_map = zeros((N, N, N)); value_map[((N*x).astype(int), (N*y).astype(int), (N*z).astype(int))] = values
