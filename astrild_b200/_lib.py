@@ -67,6 +67,15 @@ SIGNATURES = {
     "apk_bispec_count": [_vp, _vp, _sz, _vp, ct.POINTER(_d), _vp],
     "apk_bispec_measure": [_vp, _vp, _vp, _vp, _sz, _vp, _vp],
     "apk_bispec_last_ms": [_vp, ct.POINTER(ct.c_float)],
+    "apk_xi_create": [ct.POINTER(_vp), _vp, _d, _d, _d, _i, _vp, _i, _vp, _i, _i],
+    "apk_xi_destroy": [_vp],
+    "apk_xi_edges": [_vp, _vp, _i, ct.POINTER(_i)],
+    "apk_xi_scratch_bytes": [_vp, ct.POINTER(_sz)],
+    "apk_xi_grid_scale": [_vp, ct.POINTER(_d)],
+    "apk_xi_measure": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp],
+    "apk_xi_last_ms": [_vp, ct.POINTER(ct.c_float)],
+    "apk_tables_r_axis": [_i, _d, _vp],
+    "apk_tables_r_edges": [_i, _d, _d, _d, _d, _vp, _i, ct.POINTER(_i)],
     "apk_assign_grid": [_vp, _vp, _vp, _vp, _i, _vp, _i, _i64, _vp, _vp, _vp, _vp],
     "apk_gather_records": [_vp, _vp, _i64, _vp, _i, _vp],
     "apk_tables_k_axis": [_i, _d, _i, _vp],

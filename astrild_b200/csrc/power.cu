@@ -184,6 +184,29 @@ int apk_tables_k_edges(int nmesh, double boxsize, double kmin, double dk, double
     return 0;
 }
 
+int apk_tables_r_axis(int nmesh, double boxsize, double *r_host) {
+    APK_REQUIRE(nmesh >= 1 && boxsize > 0.0 && r_host, "apk_tables_r_axis: bad argument");
+    const double h = boxsize / (double)nmesh;
+    for (int i = 0; i < nmesh; ++i) r_host[i] = (double)freq_index(i, nmesh) * h;
+    return 0;
+}
+
+int apk_tables_r_edges(int nmesh, double boxsize, double rmin, double dr, double rmax, double *edges_host, int capacity,
+                       int *nedges) {
+    APK_REQUIRE(nmesh >= 1 && boxsize > 0.0 && nedges, "apk_tables_r_edges: bad argument");
+    if (!(dr > 0.0)) dr = boxsize / (double)nmesh;
+    if (!(rmax > 0.0)) rmax = boxsize / 2.0 + dr / 2.0;
+    std::vector<double> e;
+    const int n = arange(rmin, rmax, dr, e);
+    APK_REQUIRE(n >= 0, "apk_tables_r_edges: too many edges");
+    *nedges = n;
+    if (edges_host) {
+        APK_REQUIRE(capacity >= n, "apk_tables_r_edges: %d edges, room for %d", n, capacity);
+        std::memcpy(edges_host, e.data(), sizeof(double) * (size_t)n);
+    }
+    return 0;
+}
+
 int apk_tables_hermitian_weights(int nmesh, double *w_host) {
     APK_REQUIRE(nmesh >= 1 && w_host, "apk_tables_hermitian_weights: bad argument");
     for (int i = 0; i < nmesh / 2 + 1; ++i) w_host[i] = freq_index(i, nmesh) > 0 ? 2.0 : 1.0;

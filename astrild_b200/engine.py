@@ -72,6 +72,18 @@ class BispecBinning:
 
 
 @dataclass
+class XiBinning:
+    handle: ct.c_void_p
+    edges: np.ndarray
+    muedges: np.ndarray
+    ells: tuple
+    nmu: int
+    scratch_bytes: int
+    grid_scale: float            # the output grid holds grid_scale * sum w p e^{ikr} of the un-normalised fields
+    key: tuple
+
+
+@dataclass
 class KmuBinning:
     handle: ct.c_void_p
     edges: np.ndarray
@@ -107,6 +119,8 @@ class PkEngine:
             for b in self._binnings.values():
                 if isinstance(b, BispecBinning):
                     self.lib.apk_bispec_destroy(b.handle)
+                elif isinstance(b, XiBinning):
+                    self.lib.apk_xi_destroy(b.handle)
                 else:
                     (self.lib.apk_kmu_destroy if isinstance(b, KmuBinning) else self.lib.apk_binning_destroy)(b.handle)
             self._binnings.clear()
@@ -609,3 +623,78 @@ class PkEngine:
         return {"k1": k[ijl[:, 0]], "k2": k[ijl[:, 1]], "k3": k[ijl[:, 2]], "bins": ijl.astype(np.int64), "B": B,
                 "triangles": ntri[keep].copy(), "P1": P1, "P2": P2, "P3": P3, "Bshot": Bshot}
 
+    # ------------------------------------------------------------------ correlation function (FFT estimator)
+    def xi_binning(self, rmin: float = 0.0, dr: float | None = None, rmax: float | None = None, Nmu: int = 1, poles=(),
+                   los=(0.0, 0.0, 1.0), compensation: tuple | None = None, interlaced: bool = False) -> "XiBinning":
+        """Edges, (r, mu) bins and the C2R plan of a correlation function (apk_xi_create): dr defaults to L / N, rmax to
+        L / 2 + dr / 2.  Nmu == 1 without poles is the 1-D path.  Cached like the other binnings."""
+        if self.n0 != self.N:
+            raise AstrildPkError("the correlation function runs on single-GPU engines only (no slab path)")
+        ells = tuple(sorted(set([0] + [int(e) for e in poles])))
+        key = ("xi", float(rmin), None if dr is None else float(dr), None if rmax is None else float(rmax), int(Nmu), ells,
+               tuple(float(x) for x in los), compensation, bool(interlaced))
+        got = self._binnings.get(key)
+        if got is not None:
+            return got
+        rs = 0 if compensation is None else _lib.RESAMPLERS[str(compensation[0]).lower()]
+        ea = np.asarray(ells, dtype=np.int32)
+        la = np.asarray(los, dtype=np.float64)
+        handle = ct.c_void_p()
+        _lib.call("apk_xi_create", ct.byref(handle), self._plan, float(rmin), 0.0 if dr is None else float(dr),
+                  0.0 if rmax is None else float(rmax), int(Nmu), ea.ctypes.data_as(ct.c_void_p), len(ells),
+                  la.ctypes.data_as(ct.c_void_p), rs, int(bool(interlaced)))
+        try:
+            n = ct.c_int()
+            _lib.call("apk_xi_edges", handle, None, 0, ct.byref(n))
+            edges = np.empty(n.value)
+            _lib.call("apk_xi_edges", handle, edges.ctypes.data_as(ct.c_void_p), n.value, ct.byref(n))
+            need, gs = ct.c_size_t(), ct.c_double()
+            _lib.call("apk_xi_scratch_bytes", handle, ct.byref(need))
+            _lib.call("apk_xi_grid_scale", handle, ct.byref(gs))
+        except Exception:
+            self.lib.apk_xi_destroy(handle)
+            raise
+        got = XiBinning(handle, edges, np.linspace(0.0, 1.0, int(Nmu) + 1), ells, int(Nmu), need.value, gs.value, key)
+        self._binnings[key] = got
+        return got
+
+    def xi_raw(self, xb: "XiBinning", c1, c1s=None, c2=None, c2s=None, grid: torch.Tensor | None = None,
+               scratch: torch.Tensor | None = None) -> tuple:
+        """-> (grid, sums): the padded mesh holding xi on the grid (times xb.grid_scale, un-normalised fields) and the raw
+        float64 sums [3 + nell][(nedges + 1) (Nmu + 2)] = rsum, musum, count (int64 bits), ysum[ell].  The complex
+        fields are read, never modified."""
+        if grid is None:
+            grid = self.new_mesh()
+        if tuple(grid.shape) != (self.N, self.N, self.ldz) or grid.dtype != torch.float32 or not grid.is_contiguous():
+            raise AstrildPkError(f"the output grid must be a contiguous float32 mesh {(self.N, self.N, self.ldz)}")
+        if scratch is None and xb.scratch_bytes:
+            scratch = torch.empty(xb.scratch_bytes, dtype=torch.uint8, device=self.device)
+        nb = (len(xb.edges) + 1) * (xb.nmu + 2)
+        sums = torch.empty((3 + len(xb.ells), nb), dtype=torch.float64, device=self.device)
+        _lib.call("apk_xi_measure", xb.handle, _ptr(c1), _ptr(c1s), _ptr(c2), _ptr(c2s), _ptr(grid), _ptr(scratch),
+                  0 if scratch is None else scratch.numel(), _ptr(sums), self.stream)
+        return grid, sums
+
+    @staticmethod
+    def finish_xi(host: np.ndarray, xb: "XiBinning", scale: float) -> dict:
+        """Raw sums (host float64, row 2 int64 bits) -> ``r``, ``corr``, ``modes`` (and ``mu`` for Nmu > 1) of shape
+        (Nr, Nmu) and ``poles`` = {"r", "modes", "corr_<ell>"}; scale = s1 s2 / N^6 (the fields' scales)."""
+        nr1, nm2 = len(xb.edges) + 1, xb.nmu + 2
+        nsum = host[2].view(np.int64).reshape(nr1, nm2)
+        xsum, musum = host[0].reshape(nr1, nm2), host[1].reshape(nr1, nm2)
+        ysum = host[3:].reshape(-1, nr1, nm2) * scale
+        sl = slice(1, -1)
+        with np.errstate(invalid="ignore", divide="ignore"):
+            res = {"r": (xsum / nsum)[sl, sl], "mu": (musum / nsum)[sl, sl], "corr": (ysum[0] / nsum)[sl, sl],
+                   "modes": nsum[sl, sl].copy(), "edges": xb.edges, "muedges": xb.muedges}
+            n1 = nsum[sl, sl].sum(axis=-1)
+            pol = {"r": xsum[sl, sl].sum(axis=-1) / n1, "modes": n1}
+            for i, ell in enumerate(xb.ells[:ysum.shape[0]]):
+                pol["corr_%d" % ell] = ysum[i][sl, sl].sum(axis=-1) / n1
+            res["poles"] = pol
+        return res
+
+    def last_xi_ms(self, xb: "XiBinning") -> dict:
+        ms = (ct.c_float * 3)()
+        _lib.call("apk_xi_last_ms", xb.handle, ms)
+        return {"fill": ms[0], "c2r": ms[1], "bin": ms[2]}

@@ -376,3 +376,79 @@ class FFTBispectrum:
 
     def run(self):
         return self.bispectrum
+
+
+class FFTCorr:
+    """Two-point correlation function: ``FFTCorr(first, mode='1d' | '2d', Nmesh=None, BoxSize=None, second=None,
+    los=[0, 0, 1], Nmu=5, dr=None, rmin=0., rmax=None, poles=[])`` (nbodykit's signature).
+
+    The FFT estimator, the configuration-space twin of FFTPower on the same fields: with p = c1 conj(c2) (k = 0 zeroed)
+    xi(r) = Re sum_k w(k) p(k) e^{i k.r} over the stored half grid with FFTPower's Hermitian weights, i.e.
+    <delta1(x + r) delta2(x)> for normalised fields (rho_mean^2 xi for un-normalised ones); r = x1 - x2.  Binned on the
+    real grid with nbodykit's project_to_basis conventions: every grid point has weight 1, edges
+    ``arange(rmin, rmax, dr)`` with dr = L / N and rmax = L / 2 + dr / 2 by default, mu = (r . los) / |r|, wedges of |mu|
+    and multipoles (2 ell + 1) L_ell(mu) xi of the signed mu (odd ell carry the asymmetry of a cross correlation).
+
+    ``self.corr`` has ``r`` (mean |r| of the bin's grid points), ``corr``, ``modes`` (grid points) and, in 2d, ``mu``
+    with dims (r, mu); ``self.poles`` has ``r``, ``modes`` and ``corr_<ell>``.  This is a mesh estimator: good for r of a
+    few cells and up.  r = 0 is an ordinary grid point, so with rmin = 0 the first bin carries the shot-noise spike;
+    ``attrs["shotnoise"]`` is FFTPower's value and is reported, never subtracted.  Single-GPU meshes without folding;
+    the output grid and the C2R's work area must fit in free device memory.
+    """
+
+    def __init__(self, first, mode="1d", Nmesh=None, BoxSize=None, second=None, los=(0, 0, 1), Nmu=5, dr=None, rmin=0.0,
+                 rmax=None, poles=()):
+        if mode not in ("1d", "2d"):
+            raise AstrildPkError("mode must be '1d' or '2d'")
+        poles = [] if poles is None else [int(e) for e in poles]
+        Nmu = 1 if mode == "1d" else int(Nmu)
+        for m in (first, second):
+            if m is not None and getattr(m, "_fold", 0):
+                raise AstrildPkError("FFTCorr does not support folded boxes (fold > 0)")
+        eng = first._eng
+        if eng.n0 != eng.N:
+            raise AstrildPkError("FFTCorr runs on single-GPU meshes only (no slab path)")
+        if second is not None and second is not first and second._eng is not eng:
+            raise AstrildPkError("first and second must share Nmesh, BoxSize and device")
+        self.first, self.second = first, first if second is None else second
+        N, L = eng.N, eng.L
+        (c1, c1s), s1, comp1 = first._complex_fields()
+        if second is None or second is first:
+            c2 = c2s = None
+            s2 = s1
+        else:
+            (c2, c2s), s2, comp2 = second._complex_fields()
+            if (c1s is None) != (c2s is None):
+                raise AstrildPkError("first and second must both be interlaced or both not")
+            if comp1 != comp2:
+                raise AstrildPkError("first and second must use the same window compensation")
+        xb = eng.xi_binning(rmin, dr, rmax, Nmu, poles, tuple(float(x) for x in los), comp1, c1s is not None)
+        need = 4 * N * N * eng.ldz + xb.scratch_bytes
+        free = _free_device_bytes(eng.device)
+        if need > free:
+            raise AstrildPkError(f"FFTCorr needs {need} bytes of device memory for its output grid and the C2R's work "
+                                 f"area, {free} are free")
+        grid, sums = eng.xi_raw(xb, c1, c1s, c2, c2s)
+        del grid
+        res = eng.finish_xi(sums.cpu().numpy(), xb, s1 * s2 / float(N) ** 6)
+        auto = second is None or second is first
+        shot = float(getattr(first, "shotnoise", 0.0)) if auto else 0.0
+        dr_used = float(xb.edges[1] - xb.edges[0]) if len(xb.edges) > 1 else float("nan")
+        self.attrs = {"mode": mode, "Nmesh": np.array([N] * 3), "BoxSize": np.array([L] * 3), "edges": xb.edges,
+                      "dr": L / N if dr is None else dr, "rmin": rmin, "rmax": L / 2 + dr_used / 2 if rmax is None else rmax,
+                      "Nmu": Nmu, "poles": list(poles), "los": list(los), "volume": L ** 3, "shotnoise": shot}
+        if mode == "2d":
+            self.corr = BinnedStatistic(["r", "mu"], [xb.edges, xb.muedges],
+                                        {"r": res["r"], "mu": res["mu"], "corr": res["corr"], "modes": res["modes"]},
+                                        dict(self.attrs))
+        else:
+            self.corr = BinnedStatistic(["r"], [xb.edges], {"r": res["r"][:, 0], "corr": res["corr"][:, 0],
+                                                            "modes": res["modes"][:, 0]}, dict(self.attrs))
+        self.poles = None
+        if poles:
+            data = {"r": res["poles"]["r"], "modes": res["poles"]["modes"]}
+            data.update({"corr_%d" % e: res["poles"]["corr_%d" % e] for e in poles})
+            self.poles = BinnedStatistic(["r"], [xb.edges], data, dict(self.attrs))
+
+    def run(self):
+        return self.corr, self.poles

@@ -36,6 +36,22 @@ def k_edges(N: int, L: float, kmin: float = 0.0, dk: float | None = None,
     return np.arange(kmin, kmax, dk)
 
 
+def r_axis(N: int, L: float) -> np.ndarray:
+    """Displacement of storage index n of the real grid along one axis: ``freq_index(N) * (L / N)`` (minimum image;
+    -L/2 kept for even N, as in the k tables)."""
+    return freq_index(N) * (L / N)
+
+
+def r_edges(N: int, L: float, rmin: float = 0.0, dr: float | None = None,
+            rmax: float | None = None) -> np.ndarray:
+    """FFTCorr's edges: ``dr = L / N``, ``rmax = L / 2 + dr / 2``, ``arange(rmin, rmax, dr)`` (the arange of k_edges)."""
+    if dr is None:
+        dr = L / N
+    if rmax is None:
+        rmax = L / 2 + dr / 2
+    return np.arange(rmin, rmax, dr)
+
+
 def hermitian_weights(N: int) -> np.ndarray:
     """2 for stored modes with k_z > 0 (their conjugates are not stored), 1 for k_z = 0 / Nyquist."""
     nz = freq_index(N)[: N // 2 + 1]

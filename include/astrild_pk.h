@@ -226,6 +226,34 @@ int apk_bispec_measure(apk_bispec *bk, const void *c1, const void *c1s, void *sc
                        double *tsum_dev, void *stream);     /* c1 / c1s are read, never modified */
 int apk_bispec_last_ms(apk_bispec *bk, float ms[4]);       /* fill, c2r, reduction, fold (plan timing on) */
 
+/* ---- correlation function xi(r) (FFT estimator; nbodykit FFTCorr) ---------------------------------------------- */
+/* p(k) = c1 conj(c2) of the fields apk_bin_power sees (interlace-combined and divided by the window when created with
+ * interlaced / resampler), k = 0 zeroed; xi(r_n) = Re sum_{stored k} w(k) p(k) e^{i k.r_n} with FFTPower's Hermitian
+ * weights w, i.e. (1/N^3) sum_y d1(y + r_n) d2(y) for plain fields (r = x1 - x2).  Displacement index n is
+ * freq_index(n) * L / N per axis (apk_tables_r_axis).  Edges apk_tables_r_edges(N, L, rmin, dr, rmax) (dr = 0: L / N;
+ * rmax = 0: L / 2 + dr / 2); bins numpy.digitize(r^2, edges^2) with r^2 = (ra^2 + rb^2) + rz^2 from the squared table;
+ * every grid point has weight 1, and r = 0 is an ordinary point (the shot-noise spike, never subtracted).  nmu > 1 or
+ * more than one multipole: mu = (r . los) / |r| (0 at r = 0) binned by numpy.digitize(|mu|, linspace(0, 1, nmu + 1))
+ * (mu = 1 folded into the last column), multipoles (2 ell + 1) L_ell(mu) xi with signed mu; ells[0] must be 0, at most
+ * 8.  nmu == 1 with ells = {0} is the 1-D path (musum stays 0).  Single-GPU plans only.                            */
+typedef struct apk_xi apk_xi;
+int apk_xi_create(apk_xi **xi, apk_plan *plan, double rmin, double dr, double rmax, int nmu, const int *ells_host,
+                  int nell, const double *los_host /* [3] */, int resampler /* 0 = no compensation */, int interlaced);
+int apk_xi_destroy(apk_xi *xi);
+int apk_xi_edges(const apk_xi *xi, double *edges_host /* [capacity] or NULL */, int capacity, int *nedges);
+int apk_xi_scratch_bytes(const apk_xi *xi, size_t *bytes);     /* the cuFFT work area of the C2R */
+/* the output grid holds scale * sum w p e^{ikr} of the un-normalised fields: scale = 2^-round(log2 N^3)            */
+int apk_xi_grid_scale(const apk_xi *xi, double *scale);
+/* c1, c1s, c2, c2s: complex64 k-grids after apk_fft_r2c (c1s / c2s: interlaced twins, c2 / c2s NULL for an auto
+ * correlation); read, never modified.  grid_out: a padded mesh of the plan, disjoint from the inputs; on return it
+ * holds xi on the grid (times apk_xi_grid_scale, over N^6 times the fields' scales).  sums_dev: DEVICE float64
+ * [3 + nell][(nedges + 1) (nmu + 2)], OVERWRITTEN: rsum = sum |r|, musum = sum |mu|, count (int64 bits), then per
+ * multipole sum (2 ell + 1) L_ell(mu) xi of the un-normalised fields; digitize indices, the r under/overflow rows 0 and
+ * nedges are not accumulated and stay zero.                                                                         */
+int apk_xi_measure(apk_xi *xi, const void *c1, const void *c1s, const void *c2, const void *c2s, float *grid_out,
+                   void *scratch, size_t bytes, double *sums_dev, void *stream);
+int apk_xi_last_ms(apk_xi *xi, float ms[3]);                 /* fill, c2r, binning + fold (plan timing on) */
+
 /* ---- ingest (SURVEY.md section 8f, N1) ------------------------------------------------------------------- */
 /* PowerSpectrum3D._read_data's gridder (src/astrild/power_spectra/power_spectrum_3d.py:142-148):
  *   value_map = zeros((N, N, N)); value_map[((N*x).astype(int), (N*y).astype(int), (N*z).astype(int))] = values
@@ -257,6 +285,11 @@ int apk_tables_k_axis(int nmesh, double boxsize, int k_dtype, double *k_host /* 
 int apk_tables_k_edges(int nmesh, double boxsize, double kmin, double dk, double kmax,
                        double *edges_host /* [capacity] or NULL */, int capacity, int *nedges);
 int apk_tables_hermitian_weights(int nmesh, double *w_host /* [nmesh/2+1] */);
+/* displacement of storage index n on one axis: freq_index(n) * (L / N) (minimum image, -L/2 kept for even N); r edges
+ * numpy.arange(rmin, rmax, dr) with dr <= 0: L / N and rmax <= 0: L / 2 + dr / 2 (the arange of apk_tables_k_edges)  */
+int apk_tables_r_axis(int nmesh, double boxsize, double *r_host /* [nmesh] */);
+int apk_tables_r_edges(int nmesh, double boxsize, double rmin, double dr, double rmax,
+                       double *edges_host /* [capacity] or NULL */, int capacity, int *nedges);
 int apk_tables_compensation(int resampler, int interlaced, int nmesh, double *comp_host /* [nmesh] */);
 int apk_tables_interlace_phase(int nmesh, double boxsize, double *phase_host /* [nmesh] */);
 
