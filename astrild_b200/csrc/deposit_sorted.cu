@@ -302,7 +302,8 @@ brick_tile_kernel(const VT *__restrict__ vals, const unsigned int *__restrict__ 
     using T = Tile<S, PAIR>;
     constexpr int ZC = BrickZ<S, PAIR>::CELLS;
     __shared__ __align__(16) unsigned int tile[T::CELLS];
-    __shared__ float red_s[2 * (TILE_THREADS / 32)];
+    __shared__ float red_s[TILE_THREADS / 32];
+    __shared__ double red_sd[TILE_THREADS / 32];
     __shared__ long long xoff[T::PLANE_FLUSH ? 1 : T::TX];   // table flush: mesh offset of the tile's x-planes (-1: outside the slab)
     __shared__ int yoff[T::PLANE_FLUSH ? 1 : T::TY];         // ... and of its y-rows
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -323,6 +324,7 @@ brick_tile_kernel(const VT *__restrict__ vals, const unsigned int *__restrict__ 
 
         __syncthreads();                              // (persistent grids) the previous brick's flush is complete
         for (int i = tid; i < T::CELLS / 4; i += TILE_THREADS) reinterpret_cast<uint4 *>(tile)[i] = make_uint4(0u, 0u, 0u, 0u);
+        int bad_home = -1;                            // home cell of this thread's last non-finite particle (x << 16 | y << 8 | z)
         if constexpr (!T::PLANE_FLUSH) {
             if (tid < T::TX) {
                 int px = bx * BX - T::OFF + tid;
@@ -344,30 +346,33 @@ brick_tile_kernel(const VT *__restrict__ vals, const unsigned int *__restrict__ 
             float unit = 1.f, inv_unit = 1.f, mscale = 1.f;
             int frac_bits = 0;
             if constexpr (MASS) {
-                float top = 0.f, sum = 0.f;
+                // NaN / inf masses count as 0 here (the particle loop sends them to the mesh as NaN); the sum is float64:
+                // 8191 masses near FLT_MAX sum to ~3e42
+                float top = 0.f;
+                double sum = 0.0;
                 for (unsigned int p = c0 + tid; p < c1; p += TILE_THREADS) {
-                    const float a = fabsf(vals[p].m);
+                    const float m = fabsf(vals[p].m), a = m <= 3.4028235e38f ? m : 0.f;
                     top = fmaxf(top, a);
-                    sum += a;
+                    sum += (double)a;
                 }
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) {
                     top = fmaxf(top, __shfl_xor_sync(0xffffffffu, top, o));
                     sum += __shfl_xor_sync(0xffffffffu, sum, o);
                 }
-                if (lane == 0) { red_s[warp] = top; red_s[TILE_THREADS / 32 + warp] = sum; }
+                if (lane == 0) { red_s[warp] = top; red_sd[warp] = sum; }
                 __syncthreads();
-                top = red_s[0]; sum = red_s[TILE_THREADS / 32];
+                top = red_s[0]; sum = red_sd[0];
 #pragma unroll
-                for (int i = 1; i < TILE_THREADS / 32; ++i) { top = fmaxf(top, red_s[i]); sum += red_s[TILE_THREADS / 32 + i]; }
+                for (int i = 1; i < TILE_THREADS / 32; ++i) { top = fmaxf(top, red_s[i]); sum += red_sd[i]; }
                 // 2^ceil(log2(top)), clamped to normal numbers whose reciprocal is normal too
                 int e = ((__float_as_int(top) >> 23) & 0xff) + ((__float_as_int(top) & 0x7fffff) ? 1 : 0);
                 e = min(max(e, 2), 252);
                 unit = __int_as_float(e << 23);
                 inv_unit = __int_as_float((254 - e) << 23);
-                if (!(top > 0.f) || !(sum < 3.0e38f)) { unit = 1.f; inv_unit = 0.f; sum = 1.f; }   // all-zero, inf or NaN masses: nothing to add
+                if (!(top > 0.f)) { unit = 1.f; inv_unit = 0.f; sum = 1.0; }   // all-zero masses: nothing to add
                 constexpr float WMAX = (S == 3) ? 0.43f : 1.001f;
-                const float room = 2147483648.f / (WMAX * fmaxf(sum * inv_unit, 1.f));          // sum |m'| <= n, >= 1 when top > 0
+                const float room = 2147483648.f / (WMAX * fmaxf((float)(sum * (double)inv_unit), 1.f));   // sum |m'| <= n, >= 1 when top > 0
                 frac_bits = min(((__float_as_int(room) >> 23) & 0xff) - 127, 30);
                 mscale = __int_as_float((127 + frac_bits) << 23);
             } else {
@@ -437,7 +442,12 @@ brick_tile_kernel(const VT *__restrict__ vals, const unsigned int *__restrict__ 
 #pragma unroll
                     for (int a = 0; a < S; ++a) plane[a] = tile + origin + a * T::XS;
                 }
-                if (live) {
+                // A NaN or inf coordinate (its payload is NaN) or mass stays out of the integer tile, where it would
+                // spoil the brick's other particles; the thread notes its home cell and puts a NaN there once the brick
+                // is done.  Tested by comparison, never by how NaN converts to an integer (0 on the GPU, INT_MIN on x86).
+                const bool finite = fabsf(v.x) + fabsf(v.y) + fabsf(v.z) + fabsf(kz) <= 3.4028235e38f;   // kz: m 2^s / unit
+                if (live && !finite) bad_home = (hx << 16) | (hy << 8) | hz;
+                if (live && finite) {
 #pragma unroll
                     for (int a = 0; a < S; ++a)
 #pragma unroll
@@ -498,6 +508,15 @@ brick_tile_kernel(const VT *__restrict__ vals, const unsigned int *__restrict__ 
                 }
             }
             __syncthreads();
+        }
+        // this thread's (last) non-finite particle of the brick: NaN at its home cell, so that the mesh shows it.  A
+        // plain store: NaN + anything is NaN, so the REDs of other bricks cannot undo it in either order.
+        if (bad_home >= 0) {
+            int px = bx * BX + (bad_home >> 16);
+            const int py = wrap_index32(by * BY + ((bad_home >> 8) & 0xff), G.N), pz = wrap_index32(bz * ZC + (bad_home & 0xff), G.N);
+            const bool ok = G.slab ? px < G.nplanes : true;
+            if (!G.slab) px = wrap_index32(px, G.N);
+            if (ok) mesh[((long long)px * G.N + py) * G.ldz + pz] = __int_as_float(0x7fc00000);
         }
     }
 }
