@@ -74,6 +74,11 @@ SIGNATURES = {
     "apk_xi_grid_scale": [_vp, ct.POINTER(_d)],
     "apk_xi_measure": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp],
     "apk_xi_last_ms": [_vp, ct.POINTER(ct.c_float)],
+    "apk_tf_create": [ct.POINTER(_vp), _vp, _i],
+    "apk_tf_destroy": [_vp],
+    "apk_tf_scratch_bytes": [_vp, _i, ct.POINTER(_sz)],
+    "apk_tf_field": [_vp, _vp, _vp, _vp, _i, _i, _d, _vp, _i, _i64, _i, _vp, _sz, _vp, _vp],
+    "apk_tf_last_ms": [_vp, ct.POINTER(ct.c_float)],
     "apk_tables_r_axis": [_i, _d, _vp],
     "apk_tables_r_edges": [_i, _d, _d, _d, _d, _vp, _i, ct.POINTER(_i)],
     "apk_assign_grid": [_vp, _vp, _vp, _vp, _i, _vp, _i, _i64, _vp, _vp, _vp, _vp],

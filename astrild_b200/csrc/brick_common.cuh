@@ -192,6 +192,15 @@ __device__ __forceinline__ void warp_runs(unsigned int key, int lane, int &head,
     length = next - head;
 }
 
+// a brick partition of a particle set, left in the plan workspace by the count, scan and scatter kernels
+// (deposit_sorted.cu): payload records (P3 / P4) filed by brick, brick_start[nbricks + 1], the non-empty bricks
+// filled[0 .. *nfilled)
+struct BrickPartition {
+    const void *vals;
+    const unsigned int *brick_start, *filled, *nfilled;
+    BrickGrid B;
+};
+
 constexpr int PART_THREADS = 256;
 constexpr int PART_ITEMS = 4;    // consecutive particles per thread per tile
 

@@ -534,17 +534,19 @@ size_t deposit_sorted_workspace_bytes(const apk_plan *P, long long np, int with_
            2 * align256(4 * (max_bricks(P) / SCAN_SEG + 2)) + 256;
 }
 
-// mesh1 != nullptr: interlaced pair -- G is the shift-0 geometry, mesh1 gets the shift-0.5 twin
+// count, scan and scatter: the brick partition of the particles, payload and brick tables in the plan workspace.
+// marks: record the plan's deposit events 0 - 2 (apk_plan_last_deposit_ms); `who` names the caller in messages.
 template <int S, typename PT, bool SOA, bool MASS, bool PAIR>
-static int run_sorted(apk_plan *P, const void *p0, const void *p1, const void *p2, const void *mass,
-                      int mass_dtype, long long np, const DepositGeom &G, float *mesh, float *mesh1, cudaStream_t st) {
+static int partition_sorted(apk_plan *P, const void *p0, const void *p1, const void *p2, const void *mass,
+                            int mass_dtype, long long np, const DepositGeom &G, bool marks, const char *who,
+                            BrickPartition &out, cudaStream_t st) {
     using VT = typename std::conditional<MASS, P4, P3>::type;
     const BrickGrid B = make_brick_grid(G, S, PAIR);
     const size_t need = deposit_sorted_workspace_bytes(P, np, MASS, PAIR);
     // the cuFFT work areas live in the last fft_work_bytes of the same workspace and may be in use on another stream
     APK_REQUIRE(P->workspace && P->workspace_bytes >= need + P->fft_work_bytes + 256,
-                "apk_deposit: sorted path needs %zu workspace bytes (+ %zu of cuFFT work area), %zu set "
-                "(apk_plan_workspace_bytes / apk_plan_set_workspace)", need, P->fft_work_bytes + 256, P->workspace_bytes);
+                "%s: sorted path needs %zu workspace bytes (+ %zu of cuFFT work area), %zu set "
+                "(apk_plan_workspace_bytes / apk_plan_set_workspace)", who, need, P->fft_work_bytes + 256, P->workspace_bytes);
     APK_REQUIRE(np < 0xffffffffLL, "apk_deposit: more than 2^32-1 particles on one device");
     APK_REQUIRE((size_t)B.nbricks <= max_bricks(P), "apk_deposit: brick tables too small (internal)");
     unsigned char *w = (unsigned char *)P->workspace;
@@ -560,20 +562,35 @@ static int run_sorted(apk_plan *P, const void *p0, const void *p1, const void *p
 
     const long long tile = (long long)PART_THREADS * PART_ITEMS;
     const int pb = (int)std::min<long long>((np + tile - 1) / tile, (long long)P->num_sms * 8);
-    P->mark(0, st);
+    if (marks) P->mark(0, st);
     APK_CUDA(cudaMemsetAsync(counts, 0, 4 * (size_t)(B.nbricks + 1), st));
     brick_count_kernel<S, PT, SOA><<<pb, PART_THREADS, 0, st>>>((const PT *)p0, (const PT *)p1, (const PT *)p2, np, G, B, counts);
     APK_CUDA(cudaGetLastError());
-    P->mark(1, st);
+    if (marks) P->mark(1, st);
     const int nseg = (B.nbricks + SCAN_SEG - 1) / SCAN_SEG;
     brick_segsum_kernel<<<nseg, 1024, 0, st>>>(counts, B.nbricks, seg_total, seg_filled);
     APK_CUDA(cudaGetLastError());
     brick_scan_kernel<<<nseg, 1024, 0, st>>>(counts, B.nbricks, seg_total, seg_filled, brick_start, cursor, filled, counter + 1);
     APK_CUDA(cudaGetLastError());
-    P->mark(2, st);
+    if (marks) P->mark(2, st);
     brick_scatter_kernel<S, PT, SOA, MASS, VT><<<pb, PART_THREADS, 0, st>>>(
         (const PT *)p0, (const PT *)p1, (const PT *)p2, mass, mass_dtype == APK_F64, np, G, B, cursor, vals);
     APK_CUDA(cudaGetLastError());
+    out.vals = vals; out.brick_start = brick_start; out.filled = filled; out.nfilled = counter + 1; out.B = B;
+    return 0;
+}
+
+// mesh1 != nullptr: interlaced pair -- G is the shift-0 geometry, mesh1 gets the shift-0.5 twin
+template <int S, typename PT, bool SOA, bool MASS, bool PAIR>
+static int run_sorted(apk_plan *P, const void *p0, const void *p1, const void *p2, const void *mass,
+                      int mass_dtype, long long np, const DepositGeom &G, float *mesh, float *mesh1, cudaStream_t st) {
+    using VT = typename std::conditional<MASS, P4, P3>::type;
+    BrickPartition part;
+    if (int rc = partition_sorted<S, PT, SOA, MASS, PAIR>(P, p0, p1, p2, mass, mass_dtype, np, G, true, "apk_deposit", part, st))
+        return rc;
+    const BrickGrid &B = part.B;
+    const VT *vals = (const VT *)part.vals;
+    const unsigned int *brick_start = part.brick_start, *filled = part.filled, *counter = part.nfilled - 1;
 
     // one CTA per brick (CTAs beyond the number of non-empty bricks, which only the device knows, exit at once)
     const int ctas = B.nbricks;
@@ -623,6 +640,19 @@ int deposit_sorted_launch(apk_plan *P, const void *p0, const void *p1, const voi
     if (resampler == APK_TSC) return dispatch_layout<3>(P, p0, p1, p2, layout, pos_dtype, mass, mass_dtype, np, G, mesh, mesh1, st);
     // NGP has no halo and no arithmetic worth tiling: one RED per particle
     return deposit_atomic_launch(p0, p1, p2, layout, pos_dtype, mass, mass_dtype, np, resampler, G, mesh, P->num_sms, st);
+}
+
+// The NGP partition (S = 1: bricks of 24 x 8 x 32 home cells, no halo) of the Taylor-Fourier moment deposit (tf.cu):
+// the same count, scan and scatter kernels; the payload is the brick-local coordinates (+ mass), home cell = rint(l).
+int sorted_partition_ngp(apk_plan *P, const void *p0, const void *p1, const void *p2, int layout, int pos_dtype,
+                         const void *mass, int mass_dtype, long long np, const DepositGeom &G, BrickPartition &out,
+                         cudaStream_t st) {
+    const char *who = "apk_tf_field";
+#define APK_PART(PT, SOA) (mass ? partition_sorted<1, PT, SOA, true, false>(P, p0, p1, p2, mass, mass_dtype, np, G, false, who, out, st) \
+                                : partition_sorted<1, PT, SOA, false, false>(P, p0, p1, p2, mass, mass_dtype, np, G, false, who, out, st))
+    if (pos_dtype == APK_F32) return layout == APK_SOA ? APK_PART(float, true) : APK_PART(float, false);
+    return layout == APK_SOA ? APK_PART(double, true) : APK_PART(double, false);
+#undef APK_PART
 }
 
 }  // namespace apk

@@ -84,6 +84,14 @@ class XiBinning:
 
 
 @dataclass
+class TfPlan:
+    handle: ct.c_void_p
+    order: int
+    nmom: int                    # C(order + 3, 3) moment grids
+    key: tuple
+
+
+@dataclass
 class KmuBinning:
     handle: ct.c_void_p
     edges: np.ndarray
@@ -121,6 +129,8 @@ class PkEngine:
                     self.lib.apk_bispec_destroy(b.handle)
                 elif isinstance(b, XiBinning):
                     self.lib.apk_xi_destroy(b.handle)
+                elif isinstance(b, TfPlan):
+                    self.lib.apk_tf_destroy(b.handle)
                 else:
                     (self.lib.apk_kmu_destroy if isinstance(b, KmuBinning) else self.lib.apk_binning_destroy)(b.handle)
             self._binnings.clear()
@@ -698,3 +708,64 @@ class PkEngine:
         ms = (ct.c_float * 3)()
         _lib.call("apk_xi_last_ms", xb.handle, ms)
         return {"fill": ms[0], "c2r": ms[1], "bin": ms[2]}
+
+    # ------------------------------------------------------------------ Taylor-Fourier mesh (window-free delta(k))
+    def tf_plan(self, order: int = 3) -> "TfPlan":
+        """The Taylor-Fourier object of one order (apk_tf_create): coefficient tables w^a / a!.  Cached like the
+        binnings and destroyed with the engine."""
+        if self.n0 != self.N:
+            raise AstrildPkError("the Taylor-Fourier mesh runs on single-GPU engines only (no slab path)")
+        order = int(order)
+        key = ("tf", order)
+        got = self._binnings.get(key)
+        if got is not None:
+            return got
+        handle = ct.c_void_p()
+        _lib.call("apk_tf_create", ct.byref(handle), self._plan, order)
+        got = TfPlan(handle, order, (order + 1) * (order + 2) * (order + 3) // 6, key)
+        self._binnings[key] = got
+        return got
+
+    def tf_scratch_bytes(self, tp: "TfPlan", group: int) -> int:
+        need = ct.c_size_t()
+        _lib.call("apk_tf_scratch_bytes", tp.handle, int(group), ct.byref(need))
+        return need.value
+
+    def tf_field(self, tp: "TfPlan", pos, mass=None, pos_scale: float | None = None, group: int | None = None,
+                 out: torch.Tensor | None = None, scratch: torch.Tensor | None = None) -> torch.Tensor:
+        """c_TF of the particles (apk_tf_field) as the complex64 [N][N][N/2+1] view of a padded mesh (``out`` or a new
+        one), un-normalised like ``r2c``'s output.  Host particles are uploaded once.  group: moment meshes per pass
+        (default: all of them if they fit in free device memory, else as many as fit)."""
+        p0, p1, p2, layout, dt, npart, keep = self._positions(pos)
+        m = None
+        if mass is not None:
+            m = self._to_device(mass).contiguous()
+            if m.ndim != 1 or m.shape[0] != npart:
+                raise AstrildPkError("mass must have one entry per particle")
+        if out is None:
+            out = self.new_mesh()
+        if tuple(out.shape) != (self.N, self.N, self.ldz) or out.dtype != torch.float32 or not out.is_contiguous():
+            raise AstrildPkError(f"the output must be a contiguous float32 mesh {(self.N, self.N, self.ldz)}")
+        mesh_bytes = 4 * self.N * self.N * self.ldz
+        if group is None:
+            free, _total = torch.cuda.mem_get_info(self.device)
+            free += torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+            group = max(1, min(tp.nmom, int(free * 0.9) // mesh_bytes))
+        need = self.tf_scratch_bytes(tp, group)
+        if scratch is None or scratch.numel() < need:
+            scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
+        self.ensure_workspace(npart, m is not None)
+        _lib.call("apk_tf_field", tp.handle, _ptr(p0), _ptr(p1), _ptr(p2), layout,
+                  _lib.APK_F32 if dt == torch.float32 else _lib.APK_F64,
+                  float(1.0 / self.L if pos_scale is None else pos_scale), _ptr(m),
+                  _lib.APK_F32 if (m is None or m.dtype == torch.float32) else _lib.APK_F64, int(npart), int(group),
+                  _ptr(scratch), scratch.numel(), _ptr(out), self.stream)
+        # self.stream is torch's current stream on self.device, the stream the caching allocator tied `scratch`, `out`
+        # and the uploaded particles to: a block freed here is handed out again only to work queued after this call's
+        del keep
+        return torch.view_as_complex(out.view(self.N, self.N, self.Nk, 2))
+
+    def last_tf_ms(self, tp: "TfPlan") -> dict:
+        ms = (ct.c_float * 4)()
+        _lib.call("apk_tf_last_ms", tp.handle, ms)
+        return {"partition": ms[0], "tiles": ms[1], "r2c": ms[2], "combine": ms[3]}

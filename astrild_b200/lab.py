@@ -214,6 +214,71 @@ class CatalogMesh:
         return (c, cs), scale, comp
 
 
+class TaylorFourierMesh:
+    """Particles as a window-free mesh source: the Taylor-Fourier estimator of Colombi et al. (2009), POWMES' ``norder``.
+
+    ``TaylorFourierMesh(position, BoxSize, Nmesh, weight=None, order=3, normalize=True, fold=0, pos_scale=None,
+    device=None)``.  For order n, the moment grids M_alpha[h] = sum_p m_p dx^a dy^b dz^c (h = the particle's nearest grid
+    point, d = g - h, |alpha| <= n) are deposited on the device, transformed and combined into
+    c_TF(k) = sum_alpha (-i)^|alpha| (wx^a wy^b wz^c / a! b! c!) M^_alpha(k) (w = 2 pi freq_index / N): the DFT of the
+    particles themselves up to sum_p |m_p| (|w|_1 / 2)^(n+1) / (n+1)!, with no assignment window to deconvolve and no
+    aliasing beyond that.  Order 0 is the NGP paint.  The field has no interlaced twin and no compensation.
+
+    position, weight, normalize, fold and pos_scale are CatalogMesh's: 1 + delta (or rho = mass / dx^3), the box folded
+    f times onto itself (x -> 2^f x mod L, the spectrum reaching 2^f times the mesh's Nyquist frequency), amplitude and
+    ``shotnoise`` = V sum(w^2) / sum(w)^2 of the full volume.  That Poisson value is what ``attrs`` report; the TF
+    estimate's own noise floor differs from it by the factor E|T_n(w.d)|^2 (DESIGN section 10).  Single-GPU meshes only.
+    """
+
+    def __init__(self, position, BoxSize, Nmesh, weight=None, order=3, normalize=True, fold: int = 0, pos_scale=None,
+                 device=None):
+        self._fold = int(fold)
+        if self._fold < 0 or self._fold > 10:
+            raise AstrildPkError("fold must be between 0 and 10")
+        order = int(order)
+        if order < 0 or order > 4:
+            raise AstrildPkError("order must be between 0 and 4")
+        L = _box3(BoxSize)
+        self.attrs = {"BoxSize": np.array([L] * 3), "Nmesh": np.array([_nmesh(Nmesh)] * 3), "order": order,
+                      "fold": self._fold}
+        self._eng = _engine.get_engine(_nmesh(Nmesh), L / 2 ** self._fold, device)
+        if self._eng.n0 != self._eng.N:
+            raise AstrildPkError("TaylorFourierMesh runs on single-GPU meshes only (no slab path)")
+        self._pos, self._w = position, weight
+        self._order = order
+        self._normalize = bool(normalize)
+        self._pos_scale = (1.0 / L if pos_scale is None else pos_scale) * 2 ** self._fold
+        self.shotnoise = 0.0
+
+    _npart = CatalogMesh._npart
+    _shotnoise = CatalogMesh._shotnoise
+
+    def _complex_fields(self):
+        eng = self._eng
+        w, unit = self._w, 1.0
+        if w is not None and np.isscalar(w):
+            unit, w = float(w), None                  # a scalar weight scales the field (it cancels when normalised)
+        elif w is not None and isinstance(w, torch.Tensor) and w.is_cuda:
+            w, unit = eng.pow2_scaled(w)              # weights in units of 2^e (exact), see PkEngine.pow2_scaled
+        elif w is not None:
+            wa = np.asarray(w)
+            top = float(np.abs(wa).max()) if wa.size else 1.0
+            if np.isfinite(top) and top > 0.0:
+                unit = 2.0 ** round(float(np.log2(top)))
+                w = wa * wa.dtype.type(1.0 / unit) if wa.dtype in (np.float32, np.float64) else wa.astype(np.float64) / unit
+        tp = eng.tf_plan(self._order)
+        c = eng.tf_field(tp, self._pos, w, self._pos_scale)
+        if self._normalize:
+            # the k = 0 mode of c_TF is the sum of the moment-0 grid: the deposited mass (in units of `unit`)
+            total = float(c[0, 0, 0].real.item())
+            scale = eng.N ** 3 / total
+        else:
+            scale = unit / (eng.L / eng.N) ** 3 / 8.0 ** self._fold
+        scale *= 2.0 ** (1.5 * self._fold)
+        self.shotnoise = self._shotnoise()
+        return (c, None), scale, None
+
+
 class BinnedStatistic:
     """Minimal stand-in for nbodykit's BinnedStatistic: ``obj["k"]``, ``.attrs``, ``.edges``."""
 
@@ -355,7 +420,7 @@ class FFTBispectrum:
         binning = eng.binning(kmin, bk.dk, bk.kmax, comp, c1s is not None, k_dtype)
         power = eng.bin_power(binning, c1, c1s, None, None, L ** 3 * s * s / float(N) ** 6)
         del scratch
-        if isinstance(first, CatalogMesh):
+        if isinstance(first, (CatalogMesh, TaylorFourierMesh)):
             w = first._w
             S = float(first.shotnoise)
             if w is not None and not np.isscalar(w):

@@ -254,6 +254,28 @@ int apk_xi_measure(apk_xi *xi, const void *c1, const void *c1s, const void *c2, 
                    void *scratch, size_t bytes, double *sums_dev, void *stream);
 int apk_xi_last_ms(apk_xi *xi, float ms[3]);                 /* fill, c2r, binning + fold (plan timing on) */
 
+/* ---- Taylor-Fourier mesh (Colombi et al. 2009; POWMES `norder`): a window-free delta(k) ------------------------ */
+/* For order n (0..4) the C(n+3, 3) moment grids M_alpha[h] = sum_{p with home h} m_p dx^a dy^b dz^c (h = nearest grid
+ * point of g = pos * pos_scale * N, d = g - h in [-1/2, 1/2]^3, |alpha| <= n, graded order) are deposited from the
+ * sorted deposit's NGP brick partition, transformed with the plan's r2c and combined into
+ *   c_TF(k) = sum_alpha (-i)^|alpha| (wx^a wy^b wz^c / (a! b! c!)) M^_alpha(k),   w = 2 pi freq_index / N,
+ * which differs from the exact DFT sum_p m_p e^{-i w.g_p} by at most sum_p |m_p| (|w|_1 / 2)^{n+1} / (n+1)!.  Order 0
+ * is the NGP paint's r2c.  A particle with a NaN or inf coordinate or mass deposits nothing and puts NaN at its home
+ * cell of every moment grid.  Single-GPU plans only.                                                                */
+typedef struct apk_tf apk_tf;
+int apk_tf_create(apk_tf **tf, apk_plan *plan, int order);
+int apk_tf_destroy(apk_tf *tf);
+/* `group` moment meshes (padded, of the plan), nothing else: each pass deposits, transforms and combines `group`
+ * moments, so the particles are partitioned once and walked ceil(C(n+3, 3) / min(group, 8)) times                    */
+int apk_tf_scratch_bytes(const apk_tf *tf, int group, size_t *bytes);
+/* Particle arguments as in apk_deposit (DEVICE pointers); the partition payload lives in the plan workspace
+ * (apk_plan_workspace_bytes(plan, np, mass != NULL, 0)).  out_mesh: a padded mesh of the plan, disjoint from the
+ * scratch; on return it holds c_TF as complex64 [N][N][N/2+1] (un-normalised, like apk_fft_r2c's output).         */
+int apk_tf_field(apk_tf *tf, const void *p0, const void *p1, const void *p2, int layout, int pos_dtype, double pos_scale,
+                 const void *mass, int mass_dtype, int64_t np, int group, void *scratch, size_t bytes, float *out_mesh,
+                 void *stream);
+int apk_tf_last_ms(apk_tf *tf, float ms[4]);   /* partition, moment tiles, r2c, combine, summed over passes (plan timing on) */
+
 /* ---- ingest (SURVEY.md section 8f, N1) ------------------------------------------------------------------- */
 /* PowerSpectrum3D._read_data's gridder (src/astrild/power_spectra/power_spectrum_3d.py:142-148):
  *   value_map = zeros((N, N, N)); value_map[((N*x).astype(int), (N*y).astype(int), (N*z).astype(int))] = values
