@@ -131,6 +131,8 @@ int apk_plan_destroy(apk_plan *P) {
     if (P->has_fft1d) cufftDestroy(P->fft1d);
     if (P->scratch) cudaFree(P->scratch);
     if (P->ev_ready) for (auto &e : P->ev) cudaEventDestroy(e);
+    if (P->ovf_event) cudaEventDestroy(P->ovf_event);
+    if (P->ovf_host) cudaFreeHost(P->ovf_host);
     delete P;
     return 0;
 }
@@ -243,8 +245,12 @@ int apk_plan_last_deposit_ms(apk_plan *P, float ms[4]) {
     DeviceGuard guard(P->device);
     APK_CUDA(cudaEventSynchronize(P->ev[4]));
     ms[0] = ms[1] = ms[2] = 0.f;
-    if (P->dep_sorted)
+    if (P->dep_sorted && P->dep_fixed) {         // events: 0 scatter 1 scan (+ refiling) 2 = 3 tile kernels 4
+        APK_CUDA(cudaEventElapsedTime(&ms[2], P->ev[0], P->ev[1]));
+        APK_CUDA(cudaEventElapsedTime(&ms[1], P->ev[1], P->ev[2]));
+    } else if (P->dep_sorted) {                  // events: 0 count 1 scan 2 scatter 3 tile kernels 4
         for (int i = 0; i < 3; ++i) APK_CUDA(cudaEventElapsedTime(&ms[i], P->ev[i], P->ev[i + 1]));
+    }
     APK_CUDA(cudaEventElapsedTime(&ms[3], P->ev[3], P->ev[4]));
     return 0;
 }

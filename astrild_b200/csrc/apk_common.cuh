@@ -72,6 +72,12 @@ struct apk_plan {
     bool ev_ready = false;
     bool dep_timed = false;      // events of the last deposit are valid
     bool dep_sorted = false;
+    bool dep_fixed = false;      // ... and it partitioned in the fixed-slot layout (no count pass)
+    // fixed-slot partition (deposit_sorted.cu): its overflow word, copied to pinned host memory behind ovf_event and
+    // read only once that event has completed; ovf_seen: a brick overflowed, partition in two passes from then on
+    unsigned int *ovf_host = nullptr;
+    cudaEvent_t ovf_event = nullptr;
+    bool ovf_pending = false, ovf_seen = false;
 
     int mark(int i, cudaStream_t st) {
         if (!timing) return 0;

@@ -194,11 +194,16 @@ __device__ __forceinline__ void warp_runs(unsigned int key, int lane, int &head,
 
 // a brick partition of a particle set, left in the plan workspace by the count, scan and scatter kernels
 // (deposit_sorted.cu): payload records (P3 / P4) filed by brick, brick_start[nbricks + 1], the non-empty bricks
-// filled[0 .. *nfilled)
+// filled[0 .. *nfilled).
+// Fixed-slot layout (slots != 0): brick b's records are [b slots, b slots + fixed_count[b]) unless the device word
+// fixed_count[B.nbricks] is set -- then a brick held more than `slots` particles and brick_start describes the
+// partition as above.
 struct BrickPartition {
     const void *vals;
     const unsigned int *brick_start, *filled, *nfilled;
     BrickGrid B;
+    const unsigned int *fixed_count = nullptr;
+    unsigned int slots = 0;
 };
 
 constexpr int PART_THREADS = 256;

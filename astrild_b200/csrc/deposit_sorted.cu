@@ -20,6 +20,10 @@
 //                           (One array per coordinate instead of 12-byte records, round 2 call 34: the tile kernel's
 //                           loads become one wavefront each, 20.5 -> 20.2 ms, but the scatter writes three streams of
 //                           short runs: 6.4 -> 11.1 ms.  Records kept.)
+//      Fixed-slot layout (populated meshes, when the workspace holds >= TILE_FLUSH records per brick): every brick owns
+//      a fixed range of records, so the scatter runs first, without the count pass (3.1 of 46.4 ms per step of config
+//      3), and its cursors end as the counts that 2. scans.  A brick that overflows its slots makes the device refile
+//      the partition in the two-pass layout (see partition_sorted).
 //      Interlaced pair (apk_deposit_interlaced): the SAME partition and the same 12-byte payload serve both meshes --
 //      the twin's home cell is the same cell or the next one per axis, so its tile is one cell longer per axis
 //      (bricks hold one z-cell less) and its coordinates are the payload's + 0.5.  No second copies, no flags.
@@ -136,15 +140,28 @@ brick_scan_kernel(const unsigned int *__restrict__ counts, int n, const unsigned
     if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 1023) { start[n] = base + total; *nfilled = fbase + ftotal; }
 }
 
+#ifndef APK_TILE_FLUSH
+#define APK_TILE_FLUSH 8191
+#endif
+constexpr int TILE_FLUSH = APK_TILE_FLUSH;            // particles between two flushes of the tile (see the tile kernel)
+
 // float32 positions: 4 CTAs per SM (64 registers, no spills; measured 6.9 against 7.2 ms at 1024^3 with 3); float64: 3
 #ifndef APK_SCATTER_MIN_CTAS
 #define APK_SCATTER_MIN_CTAS (sizeof(PT) == 4 ? 4 : 3)
 #endif
+// Two-pass layout (slots == 0): cursor[] = brick_start[] from the scan of the counts; brick b's records end up in
+// [brick_start[b], brick_start[b + 1]).
+// Fixed-slot layout (slots != 0): brick b owns the records [b slots, (b + 1) slots); the cursors start at 0 and end as
+// the exact per-brick counts, so no count pass is needed.  A record beyond its brick's slots is not stored: it sets the
+// overflow word cursor[B.nbricks] instead, and the partition is then filed again in the two-pass layout.
+// only_if != nullptr: the kernel does nothing unless *only_if is set (that refiling, queued without a host round trip).
 template <int S, typename PT, bool SOA, bool MASS, typename VT>
 __global__ void __launch_bounds__(PART_THREADS, APK_SCATTER_MIN_CTAS)
 brick_scatter_kernel(const PT *__restrict__ p0, const PT *__restrict__ p1, const PT *__restrict__ p2,
                      const void *__restrict__ mass, int mass_f64, long long np, DepositGeom G,
-                     BrickGrid B, unsigned int *__restrict__ cursor, VT *__restrict__ vals) {
+                     BrickGrid B, unsigned int *__restrict__ cursor, VT *__restrict__ vals,
+                     unsigned int slots = 0, const unsigned int *__restrict__ only_if = nullptr) {
+    if (only_if && *only_if == 0u) return;
     const int lane = threadIdx.x & 31;
     const long long tile = (long long)PART_THREADS * PART_ITEMS;
     const long long step = (long long)gridDim.x * tile;
@@ -158,19 +175,18 @@ brick_scatter_kernel(const PT *__restrict__ p0, const PT *__restrict__ p1, const
         // Software pipeline of depth one: item k claims its slots (returning atomics, ~600 cycles) and item k-1,
         // whose slots have arrived meanwhile, is stored.
         VT pv = {};
-        unsigned int pslot = 0;
+        unsigned int pslot = 0, pkey = 0;
         int phead = 0, poffset = 0;
         bool plive = false;
 #pragma unroll
         for (int k = 0; k <= 4; ++k) {
             VT v = {};
-            unsigned int slot = 0;
+            unsigned int slot = 0, key = 0;
             int head = 0, offset = 0, length = 0;
             bool live = false;
             if (k < 4) {
                 const long long p = first + (long long)k * PART_THREADS;
                 float l[3];
-                unsigned int key;
                 brick_keys<S, PT>(cur.v + 3 * k, G, B, key, l);
                 if (p >= np) key = 0xffffffffu;
                 live = key != 0xffffffffu;
@@ -184,9 +200,14 @@ brick_scatter_kernel(const PT *__restrict__ p0, const PT *__restrict__ p1, const
             }
             if (k > 0) {
                 const unsigned int ps = __shfl_sync(0xffffffffu, pslot, phead) + poffset;
-                if (plive) vals[ps] = pv;
+                if (slots == 0u) {
+                    if (plive) vals[ps] = pv;
+                } else if (plive) {
+                    if (ps < slots) vals[(size_t)pkey * slots + ps] = pv;
+                    else cursor[B.nbricks] = 1u;
+                }
             }
-            pv = v; pslot = slot; phead = head; poffset = offset; plive = live;
+            pv = v; pslot = slot; pkey = key; phead = head; poffset = offset; plive = live;
         }
     }
 }
@@ -231,10 +252,6 @@ brick_scatter_kernel(const PT *__restrict__ p0, const PT *__restrict__ p1, const
 //   28.8 against 24.0 ms for both meshes at 1024^3: the sort's own shared-memory traffic (a returning ATOMS, three
 //   scattered STS and LDS per particle), its five barriers per chunk and the idle lanes of the shorter queues
 //   (utilisation 0.72) cost more than the conflicts.  Removed.
-#ifndef APK_TILE_FLUSH
-#define APK_TILE_FLUSH 8191
-#endif
-constexpr int TILE_FLUSH = APK_TILE_FLUSH;            // particles between two flushes of the tile
 #ifndef APK_TILE_THREADS
 #define APK_TILE_THREADS 256
 #endif
@@ -293,11 +310,15 @@ __device__ __forceinline__ void tile_home(float l, float last, float &d, int &h)
 
 // SEL: 0 = mesh 0 (or the only mesh), 1 = the interlaced twin (coordinates + 0.5, home cells one further); a template
 // parameter so that the clamps and the shift are immediates (as a kernel argument they were re-derived per particle)
+// slots != 0: a partition filed in the fixed-slot layout (brick_scatter_kernel), brick b's records are
+// [b slots, b slots + fixed_count[b]) -- unless the overflow word fixed_count[B.nbricks] is set: then the two-pass
+// refiling has run and brick_start describes it.  A brick of at most TILE_FLUSH particles is one chunk either way.
 template <int S, bool MASS, bool PAIR, int SEL, typename VT>
 __global__ void __launch_bounds__(TILE_THREADS, APK_TILE_CTAS)
 brick_tile_kernel(const VT *__restrict__ vals, const unsigned int *__restrict__ brick_start,
                   const unsigned int *__restrict__ filled, const unsigned int *__restrict__ nfilled_ptr,
-                  DepositGeom G, BrickGrid B, float *__restrict__ mesh) {
+                  DepositGeom G, BrickGrid B, float *__restrict__ mesh,
+                  const unsigned int *__restrict__ fixed_count = nullptr, unsigned int slots = 0) {
     static_assert(SEL == 0 || PAIR, "the twin exists only for the interlaced pair");
     using T = Tile<S, PAIR>;
     constexpr int ZC = BrickZ<S, PAIR>::CELLS;
@@ -315,9 +336,13 @@ brick_tile_kernel(const VT *__restrict__ vals, const unsigned int *__restrict__ 
     // time, so kernels of a higher-priority stream (the slab path's FFT / transpose of the first mesh) get SMs while
     // this one runs.
     const unsigned int nfilled = *nfilled_ptr;
+    const bool fixed = slots != 0u && fixed_count[B.nbricks] == 0u;
+    const unsigned int *bounds = fixed ? fixed_count : brick_start;
+    const unsigned int stride = fixed ? slots : 0u;
     for (unsigned int slot = blockIdx.x; slot < nfilled; slot += gridDim.x) {
         const unsigned int brick = filled[slot];
-        const unsigned int pbeg = brick_start[brick], pend = brick_start[brick + 1];
+        const unsigned int lo = bounds[brick], hi = bounds[brick + 1];
+        const unsigned int pbeg = stride ? brick * stride : lo, pend = stride ? pbeg + lo : hi;
         const int bz = brick % B.nbz;
         const int by = (brick / B.nbz) % B.nby;
         const int bx = brick / (B.nbz * B.nby);
@@ -525,58 +550,132 @@ static size_t max_bricks(const apk_plan *P) {
     return (size_t)((P->N + 3 + BX - 1) / BX) * ((P->N + BY - 1) / BY) * ((P->N + 28) / 29);
 }
 static size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
-
-// pair: the interlaced twins share one partition and one payload -- no extra room needed
-size_t deposit_sorted_workspace_bytes(const apk_plan *P, long long np, int with_mass, int /*pair*/) {
-    if (np <= 0) return 0;
-    const size_t vs = with_mass ? sizeof(P4) : sizeof(P3);
-    return align256(vs * (size_t)np) + 4 * align256(4 * (max_bricks(P) + 2)) +
-           2 * align256(4 * (max_bricks(P) / SCAN_SEG + 2)) + 256;
+// brick tables at the start of the workspace (4 x [max_bricks + 2], 2 x [segments + 2], counters), the payload after them
+static size_t table_bytes(const apk_plan *P) {
+    return 4 * align256(4 * (max_bricks(P) + 2)) + 2 * align256(4 * (max_bricks(P) / SCAN_SEG + 2)) + 256;
+}
+static size_t sorted_bytes(const apk_plan *P, size_t records, int with_mass) {
+    return table_bytes(P) + align256((with_mass ? sizeof(P4) : sizeof(P3)) * records);
 }
 
-// count, scan and scatter: the brick partition of the particles, payload and brick tables in the plan workspace.
+// Populated meshes (at least TILE_FLUSH / 2 particles per brick on average: 1024^3 particles on 1024^3 cells hold ~5400)
+// get room for twice their records: the fixed-slot partition (no count pass) then gives every brick twice the mean
+// occupancy, and only bricks more than twice as dense as the mean overflow.  The extra room stops at 2 TILE_FLUSH
+// records per brick: a set denser than that (mean occupancy near or above it) gets no more than its own records, and
+// with them no fixed-slot partition (see partition_sorted).  Sparse sets keep one record per particle and the two-pass
+// partition.  pair: the interlaced twins share one partition and one payload.
+static size_t payload_records(const apk_plan *P, long long np) {
+    const size_t n = (size_t)np, cap = 2 * max_bricks(P) * TILE_FLUSH;
+    if (max_bricks(P) * TILE_FLUSH > 2 * n) return n;
+    return std::max(n, std::min<size_t>({2 * n, cap, 0xffffffffu}));
+}
+size_t deposit_sorted_workspace_bytes(const apk_plan *P, long long np, int with_mass, int /*pair*/) {
+    if (np <= 0) return 0;
+    return sorted_bytes(P, payload_records(P, np), with_mass);
+}
+
+// Whether the fixed-slot partition overflowed at this plan's last fixed-slot deposit whose copy of the overflow word
+// has arrived (never waits): a plan that has seen a brick overflow its slots -- a clustered set -- partitions in two
+// passes from then on instead of paying for a fixed-slot scatter AND the refiling at every call.
+static int fixed_overflowed(apk_plan *P, bool &yes) {
+    if (P->ovf_pending) {
+        const cudaError_t e = cudaEventQuery(P->ovf_event);
+        if (e == cudaSuccess) {
+            P->ovf_pending = false;
+            if (*P->ovf_host) P->ovf_seen = true;
+        } else if (e == cudaErrorNotReady) {
+            (void)cudaGetLastError();                   // not an error: the copy is still queued
+        } else {
+            APK_CUDA(e);
+        }
+    }
+    yes = P->ovf_seen;
+    return 0;
+}
+
+// the brick partition of the particles, payload and brick tables in the plan workspace:
+//   fixed-slot layout (allow_fixed, the workspace has room for at least TILE_FLUSH records per brick, and the plan has
+//   not seen an overflow): scatter -> segment sums + scan of its exact counts (the list of non-empty bricks) -> the two-pass
+//   scatter from that scan, which runs only if a brick overflowed (the device decides; the tile kernel reads the same
+//   word).  No count pass.
+//   two-pass layout: count -> segment sums + scan -> scatter.
 // marks: record the plan's deposit events 0 - 2 (apk_plan_last_deposit_ms); `who` names the caller in messages.
 template <int S, typename PT, bool SOA, bool MASS, bool PAIR>
 static int partition_sorted(apk_plan *P, const void *p0, const void *p1, const void *p2, const void *mass,
-                            int mass_dtype, long long np, const DepositGeom &G, bool marks, const char *who,
-                            BrickPartition &out, cudaStream_t st) {
+                            int mass_dtype, long long np, const DepositGeom &G, bool marks, bool allow_fixed,
+                            const char *who, BrickPartition &out, cudaStream_t st) {
     using VT = typename std::conditional<MASS, P4, P3>::type;
     const BrickGrid B = make_brick_grid(G, S, PAIR);
-    const size_t need = deposit_sorted_workspace_bytes(P, np, MASS, PAIR);
+    const size_t need = sorted_bytes(P, (size_t)np, MASS);
     // the cuFFT work areas live in the last fft_work_bytes of the same workspace and may be in use on another stream
     APK_REQUIRE(P->workspace && P->workspace_bytes >= need + P->fft_work_bytes + 256,
                 "%s: sorted path needs %zu workspace bytes (+ %zu of cuFFT work area), %zu set "
                 "(apk_plan_workspace_bytes / apk_plan_set_workspace)", who, need, P->fft_work_bytes + 256, P->workspace_bytes);
     APK_REQUIRE(np < 0xffffffffLL, "apk_deposit: more than 2^32-1 particles on one device");
     APK_REQUIRE((size_t)B.nbricks <= max_bricks(P), "apk_deposit: brick tables too small (internal)");
+    // fixed-slot layout: as many slots per brick as the payload region set holds (32-bit record indices in the tile
+    // kernel), at least TILE_FLUSH and at least 1.5 times the mean occupancy -- with fewer, bricks would overflow
+    // as a rule and every such set would pay the refiling once
+    const size_t room = (P->workspace_bytes - P->fft_work_bytes - 256 - table_bytes(P)) / sizeof(VT);
+    const unsigned int slots = (unsigned int)std::min<size_t>(room, 0xffffffffu) / (unsigned int)B.nbricks;
+    bool fixed = allow_fixed && slots >= (unsigned int)TILE_FLUSH && 2 * (size_t)slots * B.nbricks >= 3 * (size_t)np;
+    if (fixed) {
+        bool seen = false;
+        if (int rc = fixed_overflowed(P, seen)) return rc;
+        fixed = !seen;
+    }
     unsigned char *w = (unsigned char *)P->workspace;
-    VT *vals = (VT *)w; w += align256(sizeof(VT) * (size_t)np);
     const size_t tab = align256(4 * (max_bricks(P) + 2));
-    unsigned int *counts = (unsigned int *)w; w += tab;
+    unsigned int *counts = (unsigned int *)w; w += tab;   // fixed-slot layout: the cursors, then the counts
     unsigned int *brick_start = (unsigned int *)w; w += tab;
     unsigned int *cursor = (unsigned int *)w; w += tab;
     unsigned int *filled = (unsigned int *)w; w += tab;
     unsigned int *seg_total = (unsigned int *)w; w += align256(4 * (max_bricks(P) / SCAN_SEG + 2));
     unsigned int *seg_filled = (unsigned int *)w; w += align256(4 * (max_bricks(P) / SCAN_SEG + 2));
     unsigned int *counter = (unsigned int *)w;          // [1] number of non-empty bricks
+    VT *vals = (VT *)((unsigned char *)P->workspace + table_bytes(P));
+    unsigned int *overflow = counts + B.nbricks;        // fixed-slot layout; zeroed with the counts
 
     const long long tile = (long long)PART_THREADS * PART_ITEMS;
     const int pb = (int)std::min<long long>((np + tile - 1) / tile, (long long)P->num_sms * 8);
+    const int nseg = (B.nbricks + SCAN_SEG - 1) / SCAN_SEG;
     if (marks) P->mark(0, st);
     APK_CUDA(cudaMemsetAsync(counts, 0, 4 * (size_t)(B.nbricks + 1), st));
-    brick_count_kernel<S, PT, SOA><<<pb, PART_THREADS, 0, st>>>((const PT *)p0, (const PT *)p1, (const PT *)p2, np, G, B, counts);
+    if (fixed) {
+        brick_scatter_kernel<S, PT, SOA, MASS, VT><<<pb, PART_THREADS, 0, st>>>(
+            (const PT *)p0, (const PT *)p1, (const PT *)p2, mass, mass_dtype == APK_F64, np, G, B, counts, vals, slots);
+    } else {
+        brick_count_kernel<S, PT, SOA><<<pb, PART_THREADS, 0, st>>>((const PT *)p0, (const PT *)p1, (const PT *)p2, np, G, B, counts);
+    }
     APK_CUDA(cudaGetLastError());
     if (marks) P->mark(1, st);
-    const int nseg = (B.nbricks + SCAN_SEG - 1) / SCAN_SEG;
     brick_segsum_kernel<<<nseg, 1024, 0, st>>>(counts, B.nbricks, seg_total, seg_filled);
     APK_CUDA(cudaGetLastError());
     brick_scan_kernel<<<nseg, 1024, 0, st>>>(counts, B.nbricks, seg_total, seg_filled, brick_start, cursor, filled, counter + 1);
     APK_CUDA(cudaGetLastError());
-    if (marks) P->mark(2, st);
-    brick_scatter_kernel<S, PT, SOA, MASS, VT><<<pb, PART_THREADS, 0, st>>>(
-        (const PT *)p0, (const PT *)p1, (const PT *)p2, mass, mass_dtype == APK_F64, np, G, B, cursor, vals);
-    APK_CUDA(cudaGetLastError());
+    if (fixed) {
+        // a brick overflowed: the counts are exact all the same, so the scan has laid out the two-pass payload
+        brick_scatter_kernel<S, PT, SOA, MASS, VT><<<pb, PART_THREADS, 0, st>>>(
+            (const PT *)p0, (const PT *)p1, (const PT *)p2, mass, mass_dtype == APK_F64, np, G, B, cursor, vals, 0u, overflow);
+        APK_CUDA(cudaGetLastError());
+        if (!P->ovf_host) {
+            APK_CUDA(cudaHostAlloc((void **)&P->ovf_host, sizeof(unsigned int), cudaHostAllocDefault));
+            APK_CUDA(cudaEventCreateWithFlags(&P->ovf_event, cudaEventDisableTiming));
+        }
+        APK_CUDA(cudaMemcpyAsync(P->ovf_host, overflow, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+        APK_CUDA(cudaEventRecord(P->ovf_event, st));
+        P->ovf_pending = true;
+        if (marks) P->mark(2, st);
+    } else {
+        if (marks) P->mark(2, st);
+        brick_scatter_kernel<S, PT, SOA, MASS, VT><<<pb, PART_THREADS, 0, st>>>(
+            (const PT *)p0, (const PT *)p1, (const PT *)p2, mass, mass_dtype == APK_F64, np, G, B, cursor, vals);
+        APK_CUDA(cudaGetLastError());
+    }
+    if (marks && P->timing) P->dep_fixed = fixed;
     out.vals = vals; out.brick_start = brick_start; out.filled = filled; out.nfilled = counter + 1; out.B = B;
+    out.fixed_count = fixed ? counts : nullptr;
+    out.slots = fixed ? slots : 0u;
     return 0;
 }
 
@@ -586,7 +685,8 @@ static int run_sorted(apk_plan *P, const void *p0, const void *p1, const void *p
                       int mass_dtype, long long np, const DepositGeom &G, float *mesh, float *mesh1, cudaStream_t st) {
     using VT = typename std::conditional<MASS, P4, P3>::type;
     BrickPartition part;
-    if (int rc = partition_sorted<S, PT, SOA, MASS, PAIR>(P, p0, p1, p2, mass, mass_dtype, np, G, true, "apk_deposit", part, st))
+    if (int rc = partition_sorted<S, PT, SOA, MASS, PAIR>(P, p0, p1, p2, mass, mass_dtype, np, G, true, true, "apk_deposit",
+                                                           part, st))
         return rc;
     const BrickGrid &B = part.B;
     const VT *vals = (const VT *)part.vals;
@@ -595,11 +695,13 @@ static int run_sorted(apk_plan *P, const void *p0, const void *p1, const void *p
     // one CTA per brick (CTAs beyond the number of non-empty bricks, which only the device knows, exit at once)
     const int ctas = B.nbricks;
     P->mark(3, st);
-    brick_tile_kernel<S, MASS, PAIR, 0, VT><<<ctas, TILE_THREADS, 0, st>>>(vals, brick_start, filled, counter + 1, G, B, mesh);
+    brick_tile_kernel<S, MASS, PAIR, 0, VT><<<ctas, TILE_THREADS, 0, st>>>(vals, brick_start, filled, counter + 1, G, B, mesh,
+                                                                           part.fixed_count, part.slots);
     APK_CUDA(cudaGetLastError());
     if constexpr (PAIR) {
         if (P->first_mesh_event) APK_CUDA(cudaEventRecord(P->first_mesh_event, st));
-        brick_tile_kernel<S, MASS, PAIR, 1, VT><<<ctas, TILE_THREADS, 0, st>>>(vals, brick_start, filled, counter + 1, G, B, mesh1);
+        brick_tile_kernel<S, MASS, PAIR, 1, VT><<<ctas, TILE_THREADS, 0, st>>>(vals, brick_start, filled, counter + 1, G, B,
+                                                                               mesh1, part.fixed_count, part.slots);
         APK_CUDA(cudaGetLastError());
     }
     P->mark(4, st);
@@ -648,8 +750,8 @@ int sorted_partition_ngp(apk_plan *P, const void *p0, const void *p1, const void
                          const void *mass, int mass_dtype, long long np, const DepositGeom &G, BrickPartition &out,
                          cudaStream_t st) {
     const char *who = "apk_tf_field";
-#define APK_PART(PT, SOA) (mass ? partition_sorted<1, PT, SOA, true, false>(P, p0, p1, p2, mass, mass_dtype, np, G, false, who, out, st) \
-                                : partition_sorted<1, PT, SOA, false, false>(P, p0, p1, p2, mass, mass_dtype, np, G, false, who, out, st))
+#define APK_PART(PT, SOA) (mass ? partition_sorted<1, PT, SOA, true, false>(P, p0, p1, p2, mass, mass_dtype, np, G, false, false, who, out, st) \
+                                : partition_sorted<1, PT, SOA, false, false>(P, p0, p1, p2, mass, mass_dtype, np, G, false, false, who, out, st))
     if (pos_dtype == APK_F32) return layout == APK_SOA ? APK_PART(float, true) : APK_PART(float, false);
     return layout == APK_SOA ? APK_PART(double, true) : APK_PART(double, false);
 #undef APK_PART

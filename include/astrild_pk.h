@@ -58,7 +58,10 @@ int apk_plan_destroy(apk_plan *plan);
 /* floats in one local mesh: n0 * N * 2*(N/2+1)                                               */
 int apk_plan_mesh_elems(const apk_plan *plan, int64_t *elems);
 /* bytes of scratch apk_deposit (sorted path, max_particles; interlaced != 0: apk_deposit_interlaced)
- * and apk_fft_r2c need                                                                         */
+ * and apk_fft_r2c need.  Populated meshes (8191 records per brick cost at most twice max_particles records) get room
+ * for twice max_particles payload records, and never more than 2 x 8191 records per brick of the mesh: a deposit into
+ * a workspace with room for at least 8191 records per brick, and 1.5 times its mean particles per brick, files its
+ * particles into fixed slots per brick without a count pass; a smaller workspace gives the two-pass partition. */
 int apk_plan_workspace_bytes(const apk_plan *plan, int64_t max_particles, int with_mass, int interlaced,
                              size_t *bytes);   /* deposit region + the cuFFT work areas of the plans made so far */
 int apk_plan_set_workspace(apk_plan *plan, void *workspace, size_t bytes);
@@ -69,9 +72,10 @@ int apk_plan_ghost_planes(const apk_plan *plan, int *n_lo, int *n_hi);
 /* ---- per-kernel timing (CUDA events recorded inside the library, on the caller's stream) ---- */
 /* on != 0: apk_deposit / apk_bin_power bracket their kernels with events.                     */
 int apk_plan_enable_timing(apk_plan *plan, int on);
-/* last apk_deposit on this plan, ms: [0] brick count pass, [1] segment sums + scan of the counts, [2] brick scatter
- * pass, [3] tile kernel(s) (sorted path; both meshes of an interlaced pair) or the atomic kernel(s).  Synchronises on
- * the last event. */
+/* last apk_deposit on this plan, ms: [0] brick count pass (0 for the fixed-slot partition, which has none), [1] segment
+ * sums + scan of the counts (fixed-slot partition: plus the two-pass refiling, which runs only if a brick held more
+ * than 8191 particles), [2] brick scatter pass, [3] tile kernel(s) (sorted path; both meshes of an interlaced pair) or
+ * the atomic kernel(s).  Synchronises on the last event. */
 int apk_plan_last_deposit_ms(apk_plan *plan, float ms[4]);
 /* last apk_bin_power on this binning, ms: [0] fused binning kernel, [1] fold of per-CTA copies  */
 int apk_binning_last_ms(apk_binning *binning, float ms[2]);
